@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the per-frame inference hot path (BASELINE.json: frames/sec, 5-view, N persons).
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--dump-outputs DIR]
 
 One step = one pass of the whole path (graph build -> GAT -> clustering -> encoder -> MLP) over one batch
 of synthetic frames: Panoptic 5-view, 1024 frames, 4 persons/frame (BASELINE.json configs[1]).
@@ -243,8 +243,14 @@ def main():
     ap.add_argument('--chunks', type=int, default=1, help='sub-batches of the end-to-end call (copy/compute overlap)')
     ap.add_argument('--latency-frames', type=int, default=200, help='single-frame calls timed for p50_frame_latency_ms')
     ap.add_argument('--cpu-kind', default='auto', choices=['auto', 'reference', 'port'],
-                    help='CPU arm: the unmodified reference under the import shims (needs baseline/_ref or /root/reference) or the oracle port')
+                    help='CPU arm: the unmodified reference under the import shims (needs its staged copy under baseline/_ref) or the oracle port')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last timed step returned as DIR/<name>.npy (rank 0; see dump_outputs)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or args.workload != 'pipeline'):
+        ap.error('--dump-outputs writes the outputs of the GPU pipeline (--impl b200 --workload pipeline)')
     warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -281,7 +287,7 @@ def main():
             return
         import torch
         gat, mlp = load_weights(args.config, cfg0)
-        n_steps = max(1, min(args.steps, 8) + args.warmup)                 # bounded: a few minutes whatever --steps says
+        n_steps = args.steps + args.warmup
         budget = max(3.0, min(20.0, 90.0 / n_steps))
         runs = cpu_reference_run(args.config, args.persons, gat, mlp, budget_s=budget, n_frames=4 * (os.cpu_count() or 1), kind=kind,
                                  repeats=n_steps + 1)[1:]           # [0] absorbs the workers' first-call costs
@@ -399,6 +405,15 @@ def main():
         barrier()
         tail_ms = float(tail[0].elapsed_time(tail[1]))
         ms = (float(job[0].elapsed_time(job[1])) + tail_ms) / args.steps
+    if args.dump_outputs and rank == 0:
+        # res = the last timed step; rows past the person count, and a frame's person rows past its own count, are unspecified
+        P = pm.PosePipeline.person_count(res)
+        n_persons, person_off = res['n_persons'].cpu().numpy(), res['person_off'].cpu().numpy()
+        person_rows = np.repeat(np.asarray(pb.head_off[:-1], np.int64) - person_off[:-1], n_persons) + np.arange(P)
+        dump_outputs(args.dump_outputs, {
+            'scores': res['scores'][:pb.n_nodes], 'person_heads': res['person_heads'].cpu().numpy()[person_rows],
+            'n_persons': n_persons, 'person_off': person_off, 'person_sk': res['person_sk'][:P],
+            'person_frame': res['person_frame'][:P], 'valid': res['valid'][:P], 'joints': res['joints'][:P]})
     gather_ok = None
     if gathered is not None and rank == 0:                       # the gathered records really hold every rank's results
         last = sharding.unpack_records(gathered[-1], [args.frames] * world, args.frames, P_cap, cfg.n_cameras, n_out)
@@ -963,6 +978,28 @@ def _timed(fn):
     t0 = time.perf_counter()
     fn()
     return time.perf_counter() - t0
+
+
+DUMP_BYTES = 60 << 20            # 64 MB in all with room for the .npy headers
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy: integers and float64 as float64 (exact), other floats as float32. The inputs
+    of a run are seeded, so two builds run with the same arguments can be compared file for file. When the arrays add up to
+    more than DUMP_BYTES, each keeps a fixed, seeded sample of its rows, listed in out_dir/<name>.rows.npy."""
+    host = {}
+    for name, a in arrays.items():
+        a = np.atleast_1d(a.detach().cpu().numpy() if hasattr(a, 'detach') else np.asarray(a))
+        host[name] = a.astype(np.float64 if a.dtype.kind in 'biu' or a.dtype == np.float64 else np.float32)
+    total = sum(a.nbytes for a in host.values())
+    keep = 1.0 if total <= DUMP_BYTES else DUMP_BYTES / (total + 8 * sum(len(a) for a in host.values()))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        if keep < 1.0:
+            rows = np.sort(np.random.default_rng(0).choice(len(a), max(1, int(len(a) * keep)), replace=False))
+            np.save(os.path.join(out_dir, name + '.rows.npy'), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def dropin_driver_loop(cfg, frames, gat_state, mlp_state):
