@@ -14,7 +14,7 @@ EXPORTS = ['b200pose_last_error', 'b200pose_version', 'b200pose_device_cc', 'b20
            'b200pose_set_debug', 'b200pose_pack_record', 'b200pose_linear_n', 'b200pose_linear_fused2', 'b200pose_encode_persons_n', 'b200pose_pack_json', 'b200pose_packed_sizes', 'b200pose_packed_copy', 'b200pose_packed_free',
            'b200pose_gat_aggregate_bwd', 'b200pose_grad_planes', 'b200pose_transpose_planes', 'b200pose_colsum', 'b200pose_fold_attention',
            'b200pose_mse_sigmoid', 'b200pose_sigmoid_bwd', 'b200pose_adam_step', 'b200pose_adam_step_dev',
-           'b200pose_gat_prepare_layer', 'b200pose_gat_attn_bias_grad', 'b200pose_residual_bwd_add']
+           'b200pose_gat_prepare_layer', 'b200pose_gat_attn_bias_grad', 'b200pose_residual_bwd_add', 'b200pose_mlp_adam_planes']
 
 
 class Cameras(C.Structure):
@@ -24,6 +24,13 @@ class Cameras(C.Structure):
                 ('sm_slot', C.c_void_p), ('pe_slot', C.c_void_p), ('kinv32', C.c_void_p),
                 ('t_cam2root32', C.c_void_p), ('k64', C.c_void_p), ('dist64', C.c_void_p), ('p64', C.c_void_p),
                 ('t_cam2root32_sm', C.c_void_p)]
+
+
+class MlpLayer(C.Structure):
+    """b200pose_mlp_layer (include/b200pose.h)."""
+    _fields_ = [('offset', C.c_int64), ('n', C.c_int32), ('k', C.c_int32), ('ld', C.c_int32),
+                ('w_hi', C.c_void_p), ('w_lo', C.c_void_p), ('ld_w', C.c_int32),
+                ('wt_hi', C.c_void_p), ('wt_lo', C.c_void_p), ('ld_wt', C.c_int32)]
 
 
 class B200PoseError(RuntimeError):
@@ -78,6 +85,7 @@ def lib():
         L.b200pose_gat_attn_bias_grad.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp, vp, vp, vp]
         L.b200pose_residual_bwd_add.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp]
         L.b200pose_adam_step_dev.argtypes = [vp, vp, vp, vp, C.c_int64, f32, f32, f32, f32, f32, vp, vp, vp]
+        L.b200pose_mlp_adam_planes.argtypes = [vp, vp, vp, vp, C.c_int64, C.POINTER(MlpLayer), i32, f32, f32, f32, f32, f32, vp, vp, vp]
         for name in EXPORTS:
             if name not in ('b200pose_last_error', 'b200pose_packed_free'):
                 getattr(L, name).restype = C.c_int32

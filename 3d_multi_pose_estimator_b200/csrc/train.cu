@@ -422,13 +422,11 @@ __global__ void adam_scalars_kernel(int* __restrict__ step, float lr, float b1, 
     scal[1] = (float)sqrt(1.0 - pow((double)b2, (double)t));
 }
 
-__global__ void __launch_bounds__(256) adam_dev_kernel(float* __restrict__ theta, const float* __restrict__ grad, float* __restrict__ m,
-                                                      float* __restrict__ v, long long n, float b1, float b2, float eps, float wd,
-                                                      const float* __restrict__ scal)
+// one element of the device-step Adam; shared by adam_dev_kernel and mlp_adam_planes_kernel so both round identically
+__device__ __forceinline__ float adam_dev_element(float* __restrict__ theta, const float* __restrict__ grad, float* __restrict__ m,
+                                                  float* __restrict__ v, size_t i, float b1, float b2, float eps, float wd,
+                                                  float step_size, float bc2_sqrt)
 {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const float step_size = scal[0], bc2_sqrt = scal[1];
     float g = grad[i];
     const float th = theta[i];
     if (wd != 0.f) g = fmaf(wd, th, g);
@@ -436,7 +434,83 @@ __global__ void __launch_bounds__(256) adam_dev_kernel(float* __restrict__ theta
     mi = mi + (g - mi) * (1.f - b1);
     vi = vi * b2 + (1.f - b2) * g * g;
     m[i] = mi; v[i] = vi;
-    theta[i] = th - step_size * (mi / (sqrtf(vi) / bc2_sqrt + eps));
+    const float out = th - step_size * (mi / (sqrtf(vi) / bc2_sqrt + eps));
+    theta[i] = out;
+    return out;
+}
+
+__global__ void __launch_bounds__(256) adam_dev_kernel(float* __restrict__ theta, const float* __restrict__ grad, float* __restrict__ m,
+                                                      float* __restrict__ v, long long n, float b1, float b2, float eps, float wd,
+                                                      const float* __restrict__ scal)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    adam_dev_element(theta, grad, m, v, (size_t)i, b1, b2, eps, wd, scal[0], scal[1]);
+}
+
+// Adam over a flat parameter buffer of stacked linear layers + the split-bf16 operand planes of every updated weight, in one
+// launch: per layer, the weight slot [n, ld] is walked in 32x32 tiles that update the parameters and write W planes [n, ld_w]
+// and (optional) W^T planes [k, ld_wt] - the transposed tile goes through shared memory so both stores are coalesced - and the
+// floats between this weight slot and the next (the bias) are updated element by element. grad == null: only the planes are
+// rebuilt from theta. Plane paddings are written as zeros (the next GEMM reads them as K padding).
+constexpr int kAdamPlanesMaxLayers = 16;
+constexpr int kAdamTailPerBlock = 1024;
+struct AdamPlanesLayer {
+    long long off, tail_end;                    // weight slot at off, then floats [off + n * ld, tail_end) (the bias)
+    int n, k, ld, ld_w, ld_wt, tiles_x, tiles;
+    __nv_bfloat16 *w_hi, *w_lo, *wt_hi, *wt_lo;
+};
+struct AdamPlanesArgs {
+    AdamPlanesLayer l[kAdamPlanesMaxLayers];
+    int blk_begin[kAdamPlanesMaxLayers + 1];
+    int n_layers;
+};
+
+__global__ void __launch_bounds__(256) mlp_adam_planes_kernel(const __grid_constant__ AdamPlanesArgs a, float* __restrict__ theta,
+                                                             const float* __restrict__ grad, float* __restrict__ m, float* __restrict__ v,
+                                                             float b1, float b2, float eps, float wd, const float* __restrict__ scal)
+{
+    __shared__ float tile[32][33];
+    int li = 0;
+    while (li + 1 < a.n_layers && (int)blockIdx.x >= a.blk_begin[li + 1]) ++li;
+    const AdamPlanesLayer& L = a.l[li];
+    const int local = (int)blockIdx.x - a.blk_begin[li];
+    const float step_size = grad ? scal[0] : 0.f, bc2_sqrt = grad ? scal[1] : 1.f;
+    if (local >= L.tiles) {                                    // ---- the floats after the weight slot (bias), element-wise
+        if (!grad) return;
+        const long long base = L.off + (long long)L.n * L.ld + (long long)(local - L.tiles) * kAdamTailPerBlock;
+        for (int t = threadIdx.x; t < kAdamTailPerBlock; t += blockDim.x)
+            if (base + t < L.tail_end) adam_dev_element(theta, grad, m, v, (size_t)(base + t), b1, b2, eps, wd, step_size, bc2_sqrt);
+        return;
+    }
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    const int c0 = (local % L.tiles_x) * 32, r0 = (local / L.tiles_x) * 32;
+    for (int i = ty; i < 32; i += 8) {
+        const int r = r0 + i, c = c0 + tx;
+        float x = 0.f;
+        if (r < L.n && c < L.ld) {
+            const size_t e = (size_t)L.off + (size_t)r * L.ld + c;
+            const float th = grad ? adam_dev_element(theta, grad, m, v, e, b1, b2, eps, wd, step_size, bc2_sqrt) : theta[e];
+            if (c < L.k) x = th;
+        }
+        if (r < L.n && c < L.ld_w) {
+            __nv_bfloat16 hi, lo;
+            split_bf16(x, hi, lo);
+            L.w_hi[(size_t)r * L.ld_w + c] = hi; L.w_lo[(size_t)r * L.ld_w + c] = lo;
+        }
+        tile[i][tx] = x;
+    }
+    if (!L.wt_hi) return;
+    __syncthreads();
+    const int r_pad = min(L.ld_wt, (L.n + 63) & ~63);
+    for (int i = ty; i < 32; i += 8) {
+        const int c = c0 + i, r = r0 + tx;                     // transposed: row c of W^T, column r
+        if (c < L.k && r < r_pad) {
+            __nv_bfloat16 hi, lo;
+            split_bf16(tile[tx][i], hi, lo);
+            L.wt_hi[(size_t)c * L.ld_wt + r] = hi; L.wt_lo[(size_t)c * L.ld_wt + r] = lo;
+        }
+    }
 }
 
 }  // namespace b200pose
@@ -565,6 +639,49 @@ B2_EXPORT int b200pose_adam_step_dev(float* theta, const float* grad, float* m, 
     B2_CHECK_LAUNCH();
     if (n == 0) return B200POSE_OK;
     adam_dev_kernel<<<(int)((n + 255) / 256), 256, 0, st>>>(theta, grad, m, v, (long long)n, beta1, beta2, eps, weight_decay, scalars_dev);
+    B2_CHECK_LAUNCH();
+    return B200POSE_OK;
+}
+
+B2_EXPORT int b200pose_mlp_adam_planes(float* theta, const float* grad, float* m, float* v, int64_t n_total,
+                                       const b200pose_mlp_layer* layers, int32_t n_layers, float lr, float beta1, float beta2,
+                                       float eps, float weight_decay, int32_t* step_dev, float* scalars_dev, void* stream)
+{
+    B2_CHECK_ARG(theta && layers && n_layers >= 1 && n_layers <= kAdamPlanesMaxLayers && n_total >= 0,
+                 "mlp_adam_planes: bad argument (1 <= n_layers <= %d)", kAdamPlanesMaxLayers);
+    if (grad) B2_CHECK_ARG(m && v && step_dev && scalars_dev, "mlp_adam_planes: an optimiser step needs m, v, step_dev and scalars_dev");
+    AdamPlanesArgs a;
+    a.n_layers = n_layers;
+    a.blk_begin[0] = 0;
+    long long blocks = 0;
+    for (int i = 0; i < n_layers; ++i) {
+        const b200pose_mlp_layer& s = layers[i];
+        B2_CHECK_ARG(s.w_hi && s.w_lo && (s.wt_hi == nullptr) == (s.wt_lo == nullptr), "mlp_adam_planes: layer %d: null W planes", i);
+        B2_CHECK_ARG(s.n >= 1 && s.k >= 1 && s.ld >= s.k && s.ld_w % 64 == 0 && s.ld_w >= s.ld,
+                     "mlp_adam_planes: layer %d: need n, k >= 1, ld >= k, ld_w a multiple of 64 >= ld", i);
+        if (s.wt_hi) B2_CHECK_ARG(s.ld_wt % 64 == 0 && s.ld_wt >= s.n, "mlp_adam_planes: layer %d: ld_wt must be a multiple of 64 >= n", i);
+        const long long end = s.offset + (long long)s.n * s.ld;
+        const long long next = i + 1 < n_layers ? layers[i + 1].offset : n_total;
+        B2_CHECK_ARG((i > 0 || s.offset == 0) && s.offset >= 0 && end <= next && next <= n_total,
+                     "mlp_adam_planes: layer %d: weight slots must be in increasing order inside [0, n_total), the first at 0", i);
+        AdamPlanesLayer& d = a.l[i];
+        d.off = s.offset; d.tail_end = next;
+        d.n = s.n; d.k = s.k; d.ld = s.ld; d.ld_w = s.ld_w; d.ld_wt = s.wt_hi ? s.ld_wt : 0;
+        const int rows = s.wt_hi ? ((s.n + 63) / 64) * 64 : s.n;
+        d.tiles_x = ceil_div(s.ld_w, 32);
+        d.tiles = d.tiles_x * ceil_div(rows, 32);
+        d.w_hi = reinterpret_cast<__nv_bfloat16*>(s.w_hi); d.w_lo = reinterpret_cast<__nv_bfloat16*>(s.w_lo);
+        d.wt_hi = reinterpret_cast<__nv_bfloat16*>(s.wt_hi); d.wt_lo = reinterpret_cast<__nv_bfloat16*>(s.wt_lo);
+        blocks += d.tiles + (grad ? (next - end + kAdamTailPerBlock - 1) / kAdamTailPerBlock : 0);
+        B2_CHECK_ARG(blocks < (1LL << 31), "mlp_adam_planes: too many tiles");
+        a.blk_begin[i + 1] = (int)blocks;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    if (grad) {
+        adam_scalars_kernel<<<1, 1, 0, st>>>(step_dev, lr, beta1, beta2, scalars_dev);
+        B2_CHECK_LAUNCH();
+    }
+    mlp_adam_planes_kernel<<<(int)blocks, 256, 0, st>>>(a, theta, grad, m, v, beta1, beta2, eps, weight_decay, scalars_dev);
     B2_CHECK_LAUNCH();
     return B200POSE_OK;
 }

@@ -10,6 +10,11 @@ the backward on csrc/train.cu + the split-bf16 tensor-core GEMM (dW = G^T X and 
 transposed planes). `GatTrainer` adds the loss and Adam kernels: one `step()` = the reference's loop body. The drop-in
 `gat2.GAT2` uses `GatGrad` under a `torch.autograd.Function`, so the reference's own loop (`loss.backward()`,
 `optimizer.step()`) trains the drop-in model unmodified.
+
+`MlpGrad` / `MlpTrainer` do the same for the pose-estimator MLP (utils/mlp.py:8-31: 9 linear layers, LeakyReLU(0.1) between),
+with a loss the caller writes in torch: the backward runs on the same GEMM and plane kernels, Adam and the refresh of every
+operand plane run as one fused launch (b200pose_mlp_adam_planes). The drop-in `mlp.PoseEstimatorMLP` uses `MlpGrad` under a
+`torch.autograd.Function`.
 """
 from __future__ import annotations
 
@@ -22,7 +27,7 @@ import torch
 from . import _lib
 from ._lib import check, ptr
 from .pipeline import Planes, PosePipeline, round_up
-from .weights import GAT_ALPHA, GAT_ACT_SLOPE
+from .weights import GAT_ALPHA, GAT_ACT_SLOPE, MLP_SLOPE
 
 
 def _ld4(n: int) -> int:
@@ -61,6 +66,74 @@ class _Buf:
         view = Planes.__new__(Planes)
         view.rows, view.cols, view.ld, view.hi, view.lo = rows, cols, ws.ld, ws.hi, ws.lo
         return view
+
+
+class _FlatParams:
+    """Parameters in one flat fp32 buffer `theta` (gradients in `grad`), addressed through `slots`: key -> (offset, rows, cols, ld)."""
+
+    def view(self, flat: torch.Tensor, key: str, padded: bool = False) -> torch.Tensor:
+        off, rows, cols, ld = self.slots[key]
+        t = flat[off: off + rows * ld].view(rows, ld)
+        return t if padded else t[:, :cols]
+
+    def _shape(self, key, t):
+        """the reference's tensor shapes: biases [n], weights [out, in]"""
+        return t.reshape(-1) if key.endswith('bias') else t
+
+    def load_state(self, state: Dict[str, torch.Tensor]):
+        for key in self.slots:
+            src = state[key].detach().to(self.device, torch.float32)
+            self.view(self.theta, key).copy_(src.reshape(self.slots[key][1], self.slots[key][2]))
+        self.refresh_weights()
+
+    def state_dict(self) -> Dict[str, torch.Tensor]:
+        return {key: self._shape(key, self.view(self.theta, key)).clone() for key in self.slots}
+
+    def grads(self) -> Dict[str, torch.Tensor]:
+        return {key: self._shape(key, self.view(self.grad, key)) for key in self.slots}
+
+    def _linear(self, a: Planes, m, w: Planes, n, k, out: torch.Tensor):
+        """out [m, n] fp32 = A W^T without bias or activation: the dW and dX products of a backward"""
+        self.launches += 1
+        check(self.L.b200pose_linear(ptr(a.hi), ptr(a.lo), a.ld, ptr(w.hi), ptr(w.lo), w.ld, None, m, n, k, 1.0, 1.0,
+                                     ptr(out), out.stride(0), None, None, 0, 0, self.pipe._stream()), 'linear (backward)')
+
+
+class _StepGraphs:
+    """Captured optimisation steps of a trainer, one CUDA graph per input shape key, least recently used first and at most
+    `max_cached` of them. A workspace re-allocation (buf.gen changed) drops them all: the graphs hold the old addresses."""
+
+    def _init_graphs(self, max_cached: int = 64):
+        self._graphs = collections.OrderedDict()
+        self.max_cached = max_cached
+
+    def _cached_step(self, key, buf: _Buf):
+        ent = self._graphs.get(key)
+        if ent is not None and ent['gen'] != buf.gen:
+            self._graphs.clear()
+            ent = None
+        if ent is not None:
+            self._graphs.move_to_end(key)
+        return ent
+
+    def _capture_step(self, key, ent: dict, buf: _Buf, device, enqueue):
+        """Captures enqueue() (whose workspaces an eager run has already sized) on a side stream into ent['graph']."""
+        ent['gen'] = buf.gen
+        torch.cuda.synchronize(device)
+        graph = torch.cuda.CUDAGraph()
+        side = torch.cuda.Stream(device)
+        side.wait_stream(torch.cuda.current_stream(device))
+        with torch.cuda.stream(side):
+            with torch.cuda.graph(graph, stream=side):
+                enqueue()
+        torch.cuda.current_stream(device).wait_stream(side)
+        if ent['gen'] != buf.gen:
+            raise RuntimeError('%s.step_captured: a workspace was allocated during the capture' % type(self).__name__)
+        ent['graph'] = graph
+        self._graphs[key] = ent
+        while len(self._graphs) > self.max_cached:
+            self._graphs.popitem(last=False)
+        return ent
 
 
 def param_layout(shapes: Dict[str, tuple], residual: bool = False):
@@ -113,7 +186,7 @@ def param_layout(shapes: Dict[str, tuple], residual: bool = False):
     return layers, slots, off
 
 
-class GatGrad:
+class GatGrad(_FlatParams):
     """Forward with saved activations + backward of the skeleton-matching GAT (no dropout: train_skeleton_matching.py:46-48).
     residual=True: the model was built with residual connections (gat2.py:43-48, 70-75; the shipped configuration has none)."""
 
@@ -144,31 +217,12 @@ class GatGrad:
         self.load_state(state)
 
     # ------------------------------------------------------------------ parameters
-    def view(self, flat: torch.Tensor, key: str, padded: bool = False) -> torch.Tensor:
-        off, rows, cols, ld = self.slots[key]
-        t = flat[off: off + rows * ld].view(rows, ld)
-        return t if padded else t[:, :cols]
-
     def _shape(self, key, t):
         """the reference's tensor shapes: attn_* [H, D, 1], biases [n], weights [out, in]"""
         if key.endswith('attn_l') or key.endswith('attn_r'):
             l = int(key.split('.')[1])
             return t.reshape(self.layers[l]['heads'], self.layers[l]['dim'], 1)
-        if key.endswith('bias'):
-            return t.reshape(-1)
-        return t
-
-    def load_state(self, state: Dict[str, torch.Tensor]):
-        for key in self.slots:
-            src = state[key].detach().to(self.device, torch.float32)
-            self.view(self.theta, key).copy_(src.reshape(self.slots[key][1], self.slots[key][2]))
-        self.refresh_weights()
-
-    def state_dict(self) -> Dict[str, torch.Tensor]:
-        return {key: self._shape(key, self.view(self.theta, key)).clone() for key in self.slots}
-
-    def grads(self) -> Dict[str, torch.Tensor]:
-        return {key: self._shape(key, self.view(self.grad, key)) for key in self.slots}
+        return super()._shape(key, t)
 
     def refresh_weights(self):
         """The operand planes of every projection, from the flat parameters: W1, W1^T, [W2 ; attention folds] and W2^T
@@ -222,11 +276,6 @@ class GatGrad:
         return scores[:N, 0]
 
     # ------------------------------------------------------------------ backward
-    def _linear(self, a: Planes, m, w: Planes, n, k, out: torch.Tensor):
-        self.launches += 1
-        check(self.L.b200pose_linear(ptr(a.hi), ptr(a.lo), a.ld, ptr(w.hi), ptr(w.lo), w.ld, None, m, n, k, 1.0, 1.0,
-                                     ptr(out), out.stride(0), None, None, 0, 0, self.pipe._stream()), 'linear (backward)')
-
     def backward(self, dlogit: torch.Tensor):
         """dlogit [N] fp32 = gradient of the loss w.r.t. the last layer's output (before the sigmoid). Fills self.grad."""
         if self.cache is None:
@@ -291,7 +340,7 @@ class GatGrad:
                 d, ld_d = dx, dx.stride(0)
 
 
-class GatTrainer:
+class GatTrainer(_StepGraphs):
     """One `step()` = the loop body of train_skeleton_matching.py:166-181 on a batch of training graphs.
 
     `step()` enqueues the ~125 launches of a step one by one; `step_captured()` replays the same step as ONE CUDA graph per batch
@@ -312,8 +361,7 @@ class GatTrainer:
         self.adam_scalars = torch.zeros(2, dtype=torch.float32, device=dev)
         self.loss = torch.zeros(1, dtype=torch.float32, device=dev)
         self.last_scores = None
-        self._graphs = collections.OrderedDict()        # captured steps, least recently used first
-        self.max_cached = 64
+        self._init_graphs()
 
     def features(self, db) -> Planes:
         """ndata['h'] of the batch as GEMM operand planes (the reference feeds the dense N x F matrix, :171-176)"""
@@ -353,10 +401,7 @@ class GatTrainer:
             x0 = self.features(db)
         M = int(indices.shape[0])
         key = (db.n_frames, db.n_heads, db.n_nodes, db.n_edges, M, db.max_heads, db.max_enodes, bool(getattr(g, 'general', False)), x0.ld)
-        ent = self._graphs.get(key)
-        if ent is not None and ent['gen'] != self.net.buf.gen:
-            self._graphs.clear()
-            ent = None
+        ent = self._cached_step(key, self.net.buf)
         if ent is None:
             self.pipe.wait_graph(g)
             self._enqueue(db, g, indices, labels, x0, update=False)                 # sizes every workspace; no parameter changes
@@ -367,23 +412,10 @@ class GatTrainer:
             sg.row_ptr, sg.col, sg.general, sg.pending = clone(g.row_ptr), clone(g.col), bool(getattr(g, 'general', False)), None
             sx = Planes.__new__(Planes)
             sx.rows, sx.cols, sx.ld, sx.hi, sx.lo = x0.rows, x0.cols, x0.ld, clone(x0.hi), clone(x0.lo)
-            ent = dict(db=sdb, g=sg, x0=sx, idx=clone(indices), lab=clone(labels), gen=self.net.buf.gen)
-            torch.cuda.synchronize(self.pipe.device)
-            graph = torch.cuda.CUDAGraph()
-            side = torch.cuda.Stream(self.pipe.device)
-            side.wait_stream(torch.cuda.current_stream(self.pipe.device))
-            with torch.cuda.stream(side):
-                with torch.cuda.graph(graph, stream=side):
-                    self._enqueue(sdb, sg, ent['idx'], ent['lab'], sx, update=True)
-            torch.cuda.current_stream(self.pipe.device).wait_stream(side)
-            if ent['gen'] != self.net.buf.gen:
-                raise RuntimeError('GatTrainer.step_captured: a workspace was allocated during the capture')
-            ent['graph'] = graph
-            self._graphs[key] = ent
-            while len(self._graphs) > self.max_cached:
-                self._graphs.popitem(last=False)
+            ent = dict(db=sdb, g=sg, x0=sx, idx=clone(indices), lab=clone(labels))
+            self._capture_step(key, ent, self.net.buf, self.pipe.device,
+                               lambda: self._enqueue(sdb, sg, ent['idx'], ent['lab'], sx, update=True))
         else:
-            self._graphs.move_to_end(key)
             ent['db'].head_off.copy_(db.head_off, non_blocking=True)
             ent['db'].node_off.copy_(db.node_off, non_blocking=True)
             ent['g'].row_ptr.copy_(g.row_ptr, non_blocking=True)
@@ -395,4 +427,205 @@ class GatTrainer:
         ent['graph'].replay()
         self.t += 1
         self.last_scores = self.net.cache['scores'][: db.n_nodes, 0]
+        return self.loss
+
+
+# ====================================================================================================== pose-estimator MLP
+MLP_LAYER_INDICES = tuple(range(1, 18, 2))          # nn.Sequential positions of the 9 projections (utils/mlp.py:10-28)
+
+
+def mlp_param_layout(shapes: Dict[str, tuple]):
+    """Flat fp32 layout of PoseEstimatorMLP's parameters from the shapes of a reference state dict (keys
+    `layers.{1,3,...,17}.{weight,bias}`). Returns (layers, slots, n_floats): per layer its widths (n out, k in), and per key
+    (offset, rows, cols, ld) with ld = cols rounded up to 4 floats, each weight slot followed by its layer's bias slot: every row
+    starts 16-byte aligned, so the dW GEMMs store straight into the gradient buffer, and one flat range covers the optimiser
+    step. The widths come from the weights, so any input width (252 * cameras) works; they must chain layer to layer."""
+    want = {'layers.%d.%s' % (j, w) for j in MLP_LAYER_INDICES for w in ('weight', 'bias')}
+    extra = sorted(set(shapes) - want)
+    if extra:
+        raise ValueError('MlpGrad: keys outside layers.{1,3,...,17}.{weight,bias}: %s' % extra)
+    layers, slots, off = [], {}, 0
+    for i, j in enumerate(MLP_LAYER_INDICES):
+        pre = 'layers.%d.' % j
+        if pre + 'weight' not in shapes or pre + 'bias' not in shapes:
+            raise ValueError('MlpGrad: layer %s needs a weight and a bias (utils/mlp.py builds nn.Linear with bias=True)' % pre)
+        w, b = tuple(shapes[pre + 'weight']), tuple(shapes[pre + 'bias'])
+        if len(w) != 2 or b != (w[0],) or (layers and w[1] != layers[-1]['n']):
+            raise ValueError('MlpGrad: %sweight %s, bias %s do not chain to the previous layer' % (pre, w, b))
+        n, k = w
+        slots[pre + 'weight'] = (off, n, k, _ld4(k))
+        off += n * _ld4(k)
+        slots[pre + 'bias'] = (off, 1, n, _ld4(n))
+        off += _ld4(n)
+        layers.append(dict(n=n, k=k))
+    return layers, slots, off
+
+
+class MlpGrad(_FlatParams):
+    """Forward with saved activations + backward of PoseEstimatorMLP (utils/mlp.py:8-31). The forward keeps every layer's input
+    as operand planes in a buffer of its own; the backward goes layer by layer from the last: G = dY * LeakyReLU'(Y) (the sign
+    of the stored activated planes; the last layer is linear) as planes in both layouts, d bias = column sums of G,
+    dW = G^T X into the gradient slot, dX = G W on the W^T planes (not for the first layer)."""
+
+    def __init__(self, pipe: PosePipeline, state: Dict[str, torch.Tensor], slope: float = MLP_SLOPE):
+        self.pipe = pipe
+        self.L = pipe.L
+        self.device = pipe.device
+        self.slope = float(slope)
+        self.layers, self.slots, self.n_flat = mlp_param_layout({k: tuple(v.shape) for k, v in state.items()})
+        with torch.cuda.device(self.device):
+            self.theta = torch.zeros(self.n_flat, dtype=torch.float32, device=self.device)
+            self.grad = torch.zeros(self.n_flat, dtype=torch.float32, device=self.device)
+            self.buf = _Buf(self.device)
+            for i, lay in enumerate(self.layers):
+                lay['w'] = Planes(lay['n'], lay['k'], self.device)
+                lay['wt'] = Planes(lay['k'], lay['n'], self.device) if i > 0 else None         # dX of the first layer is not needed
+        table = []
+        for i, lay in enumerate(self.layers):
+            off, n, k, ld = self.slots['layers.%d.weight' % MLP_LAYER_INDICES[i]]
+            w, wt = lay['w'], lay['wt']
+            table.append(_lib.MlpLayer(off, n, k, ld, w.hi.data_ptr(), w.lo.data_ptr(), w.ld,
+                                       wt.hi.data_ptr() if wt else None, wt.lo.data_ptr() if wt else None, wt.ld if wt else 0))
+        self._table = (_lib.MlpLayer * len(table))(*table)
+        self.cache = None
+        self.cache_token = None
+        self.launches = 0
+        self.load_state(state)
+
+    @property
+    def n_out(self) -> int:
+        return self.layers[-1]['n']
+
+    def adam_planes(self, grad, m=None, v=None, lr=0.0, betas=(0.0, 0.0), eps=0.0, weight_decay=0.0, t_dev=None, scalars=None):
+        """b200pose_mlp_adam_planes: one Adam step over theta with `grad` and the refresh of every operand plane, in one launch
+        after the scalar kernel; grad=None rebuilds the planes from theta only."""
+        check(self.L.b200pose_mlp_adam_planes(ptr(self.theta), ptr(grad), ptr(m), ptr(v), self.n_flat, self._table, len(self.layers),
+                                              lr, betas[0], betas[1], eps, weight_decay, ptr(t_dev), ptr(scalars), self.pipe._stream()),
+              'mlp_adam_planes')
+        self.launches += 1 if grad is None else 2
+
+    def refresh_weights(self):
+        self.adam_planes(None)
+
+    def forward(self, x: torch.Tensor) -> torch.Tensor:
+        """x [P, in] fp32 (contiguous rows) -> the MLP output [P, n_out] (a view of a workspace); keeps what backward() needs."""
+        pipe, P = self.pipe, int(x.shape[0])
+        if P < 1 or x.dim() != 2 or x.shape[1] != self.layers[0]['k'] or x.stride(1) != 1 or x.dtype != torch.float32:
+            raise ValueError('MlpGrad.forward: x must be fp32 [P >= 1, %d] with unit column stride, got %s %s'
+                             % (self.layers[0]['k'], x.dtype, tuple(x.shape)))
+        xp = self.buf.p('x0', P, x.shape[1])
+        check(self.L.b200pose_split_planes(ptr(x), P, x.shape[1], x.stride(0), ptr(xp.hi), ptr(xp.lo), xp.ld, pipe._stream()), 'split_planes')
+        self.launches += 1
+        xs = [xp]
+        for i, lay in enumerate(self.layers):
+            bias = self.view(self.theta, 'layers.%d.bias' % MLP_LAYER_INDICES[i])
+            if i == len(self.layers) - 1:
+                out = self.buf.f('out', P, _ld4(lay['n']))
+                pipe.linear(xs[-1], P, lay['w'], bias, lay['n'], lay['k'], 1.0, out_f32=out)
+            else:
+                y = self.buf.p('a_%d' % i, P, lay['n'])
+                pipe.linear(xs[-1], P, lay['w'], bias, lay['n'], lay['k'], self.slope, out_planes=y)
+                xs.append(y)
+        self.cache = dict(xs=xs, P=P)                     # (the projections' launches are counted by the pipeline)
+        return out[:P, : self.n_out]
+
+    def backward(self, dy: torch.Tensor):
+        """dy [P, n_out] fp32 (unit column stride) = gradient of the loss w.r.t. the output of the last forward. Fills self.grad."""
+        if self.cache is None:
+            raise RuntimeError('MlpGrad.backward without a forward')
+        L, s, P, xs = self.L, self.pipe._stream(), self.cache['P'], self.cache['xs']
+        if tuple(dy.shape) != (P, self.n_out) or dy.stride(1) != 1 or dy.dtype != torch.float32:
+            raise ValueError('MlpGrad.backward: dy must be fp32 [%d, %d] with unit column stride' % (P, self.n_out))
+        d, ld_d = dy, dy.stride(0)
+        for i in range(len(self.layers) - 1, -1, -1):
+            lay, pre = self.layers[i], 'layers.%d.' % MLP_LAYER_INDICES[i]
+            n, k, x = lay['n'], lay['k'], xs[i]
+            mask = xs[i + 1] if i + 1 < len(self.layers) else None              # the activated output of this layer
+            G = self.buf.p('G_%d' % i, P, n) if i > 0 else None
+            GT = self.buf.p('GT_%d' % i, n, P)
+            check(L.b200pose_grad_planes(ptr(d), P, n, ld_d, ptr(mask.hi) if mask else None, mask.ld if mask else 0, self.slope,
+                                         ptr(d) if mask else None, ld_d if mask else 0,
+                                         ptr(G.hi) if G else None, ptr(G.lo) if G else None, G.ld if G else 0,
+                                         ptr(GT.hi), ptr(GT.lo), GT.ld, s), 'grad_planes')
+            check(L.b200pose_colsum(ptr(d), P, n, ld_d, None, 0, 1, ptr(self.view(self.grad, pre + 'bias')), s), 'colsum')
+            xT = self.buf.p('xT_%d' % i, k, P)
+            check(L.b200pose_transpose_planes(ptr(x.hi), ptr(x.lo), P, k, x.ld, ptr(xT.hi), ptr(xT.lo), xT.ld, s), 'transpose_planes')
+            self.launches += 3
+            self._linear(GT, n, xT, k, P, self.view(self.grad, pre + 'weight', padded=True))       # dW = G^T X
+            if i > 0:
+                dx = self.buf.f('dx_%d' % i, P, _ld4(k))
+                self._linear(G, P, lay['wt'], k, n, dx)                                           # dX = G W
+                d, ld_d = dx, dx.stride(0)
+
+
+def _rows(x: torch.Tensor, device) -> torch.Tensor:
+    """nn.Flatten + fp32 + contiguous rows on the device (the MLP's input as the GEMM reads it)"""
+    return x.reshape(x.shape[0], -1).to(device, torch.float32).contiguous()
+
+
+class MlpTrainer(_StepGraphs):
+    """One `step()` = forward, the caller's torch loss on the joints and its gradient, backward, Adam, operand-plane refresh.
+    Adam's defaults are torch.optim.Adam's. `step_captured()` replays the same step, the caller's loss included, as ONE CUDA
+    graph per input shape (and loss function / arguments signature)."""
+
+    def __init__(self, pipe: PosePipeline, state: Dict[str, torch.Tensor], lr: float = 1e-3, betas: Sequence[float] = (0.9, 0.999),
+                 eps: float = 1e-8, weight_decay: float = 0.0, slope: float = MLP_SLOPE):
+        self.pipe = pipe
+        self.net = MlpGrad(pipe, state, slope)
+        self.lr, self.betas, self.eps, self.weight_decay = float(lr), (float(betas[0]), float(betas[1])), float(eps), float(weight_decay)
+        dev = pipe.device
+        self.m = torch.zeros(self.net.n_flat, dtype=torch.float32, device=dev)
+        self.v = torch.zeros(self.net.n_flat, dtype=torch.float32, device=dev)
+        self.t = 0                                                            # host mirror of the device-side step count
+        self.t_dev = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.adam_scalars = torch.zeros(2, dtype=torch.float32, device=dev)
+        self.loss = torch.zeros(1, dtype=torch.float32, device=dev)
+        self.last_joints = None
+        self._init_graphs()
+
+    def _enqueue(self, x, loss_fn, args, update):
+        net = self.net
+        out = net.forward(x)
+        joints = out.detach().requires_grad_(True)
+        with torch.enable_grad():
+            loss = loss_fn(joints, *args)
+            (dj,) = torch.autograd.grad(loss, joints)
+        self.loss.copy_(loss.detach().reshape(1))
+        net.backward(dj.contiguous())
+        if update:
+            net.adam_planes(net.grad, self.m, self.v, self.lr, self.betas, self.eps, self.weight_decay, self.t_dev, self.adam_scalars)
+        self.last_joints = out
+
+    def step(self, x: torch.Tensor, loss_fn, *args, update: bool = True):
+        """x [P, ...] MLP inputs (flattened per row); loss_fn(joints [P, n_out], *args) -> scalar tensor, plain torch code.
+        Returns the loss as a device scalar (the step itself does not synchronise)."""
+        self._enqueue(_rows(x, self.pipe.device), loss_fn, args, update)
+        if update:
+            self.t += 1
+        return self.loss
+
+    def step_captured(self, x: torch.Tensor, loss_fn, *args):
+        """step() as one CUDA-graph replay. The first call for a key (input shape, loss function, tensor arguments' shapes and
+        dtypes, other arguments by value) runs one eager forward + backward to size the workspaces and captures the step on
+        static copies of x and the tensor arguments; later calls copy their inputs there and replay. loss_fn must be capturable
+        (no host synchronisation). A workspace re-allocation (a larger batch) drops the graphs."""
+        x = _rows(x, self.pipe.device)
+        sig = lambda a: ('tensor', tuple(a.shape), a.dtype, a.device) if torch.is_tensor(a) else \
+            (a if isinstance(a, (int, float, str, bool, type(None))) else ('object', id(a)))
+        key = (tuple(x.shape), id(loss_fn)) + tuple(sig(a) for a in args)
+        ent = self._cached_step(key, self.net.buf)
+        if ent is None:
+            self._enqueue(x, loss_fn, args, update=False)                        # sizes every workspace; no parameter changes
+            sx = x.clone()
+            sargs = [a.clone() if torch.is_tensor(a) else a for a in args]
+            ent = dict(x=sx, args=sargs, fn=loss_fn, held=args)                  # holding fn / args keeps their ids unique
+            self._capture_step(key, ent, self.net.buf, self.pipe.device, lambda: self._enqueue(sx, loss_fn, sargs, update=True))
+        else:
+            ent['x'].copy_(x, non_blocking=True)
+            for st, a in zip(ent['args'], args):
+                if torch.is_tensor(a):
+                    st.copy_(a, non_blocking=True)
+        ent['graph'].replay()
+        self.t += 1
+        self.last_joints = self.net.buf.f('out', x.shape[0], _ld4(self.net.n_out))[: x.shape[0], : self.net.n_out]
         return self.loss

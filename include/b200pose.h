@@ -339,6 +339,27 @@ int b200pose_adam_step(float* theta, const float* grad, float* m, float* v, int6
 int b200pose_adam_step_dev(float* theta, const float* grad, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
                            float eps, float weight_decay, int32_t* step_dev, float* scalars_dev, void* stream);
 
+/* One linear layer of a flat parameter buffer for b200pose_mlp_adam_planes: the weight [n, k] at theta[offset], rows ld >= k
+ * floats apart; its split-bf16 operand planes W [n, ld_w] (ld_w a multiple of 64, >= ld) and, unless wt_hi is null, W^T
+ * [k, ld_wt] (ld_wt a multiple of 64, >= n). */
+typedef struct {
+    int64_t offset;
+    int32_t n, k, ld;
+    uint16_t *w_hi, *w_lo;
+    int32_t ld_w;
+    uint16_t *wt_hi, *wt_lo;
+    int32_t ld_wt;
+} b200pose_mlp_layer;
+/* b200pose_adam_step_dev over theta[0, n_total) (bit-identical theta, m, v, *step_dev and scalars_dev) fused with the refresh of
+ * every layer's operand planes from the updated weights, in one launch after the scalar kernel (PoseEstimatorMLP, utils/mlp.py:8-31,
+ * trained with torch.optim.Adam). The weight slots come in increasing offset order, the first at 0; the floats between a weight
+ * slot and the next one (or n_total) - the layer's bias - are updated too. Plane paddings (columns [k, ld_w) of W, columns
+ * [n, round_up(n, 64)) of W^T) are written as zeros. grad == null: planes only, from theta as it is (theta, m, v, lr ... and the
+ * step count are not touched; m, v, step_dev, scalars_dev may be null). At most 16 layers. */
+int b200pose_mlp_adam_planes(float* theta, const float* grad, float* m, float* v, int64_t n_total,
+                             const b200pose_mlp_layer* layers, int32_t n_layers, float lr, float beta1, float beta2,
+                             float eps, float weight_decay, int32_t* step_dev, float* scalars_dev, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Host-side frame packer (no GPU work): the reference's frame JSON - a list of frames
  * {camera: [json.dumps([skeleton, ...]), timestamp, ...]} as read by test/metrics_from_model.py:117-191, or one such
