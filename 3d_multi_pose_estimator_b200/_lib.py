@@ -12,8 +12,8 @@ EXPORTS = ['b200pose_last_error', 'b200pose_version', 'b200pose_device_cc', 'b20
            'b200pose_node_features', 'b200pose_linear', 'b200pose_split_planes', 'b200pose_gat_aggregate', 'b200pose_gat_aggregate_res',
            'b200pose_cluster', 'b200pose_cluster_pairs', 'b200pose_build_graph_pairs', 'b200pose_encode_persons', 'b200pose_triangulate', 'b200pose_gather_persons',
            'b200pose_set_debug', 'b200pose_pack_record', 'b200pose_linear_n', 'b200pose_linear_fused2', 'b200pose_encode_persons_n', 'b200pose_pack_json', 'b200pose_packed_sizes', 'b200pose_packed_copy', 'b200pose_packed_free',
-           'b200pose_gat_aggregate_bwd', 'b200pose_grad_planes', 'b200pose_transpose_planes', 'b200pose_colsum', 'b200pose_fold_attention',
-           'b200pose_mse_sigmoid', 'b200pose_sigmoid_bwd', 'b200pose_adam_step', 'b200pose_adam_step_dev',
+           'b200pose_gat_aggregate_bwd', 'b200pose_grad_planes', 'b200pose_transpose_planes', 'b200pose_colsum',
+           'b200pose_mse_sigmoid', 'b200pose_sigmoid_bwd', 'b200pose_adam_step_dev',
            'b200pose_gat_prepare_layer', 'b200pose_gat_attn_bias_grad', 'b200pose_residual_bwd_add', 'b200pose_mlp_adam_planes']
 
 
@@ -77,10 +77,8 @@ def lib():
         L.b200pose_grad_planes.argtypes = [vp, i32, i32, i32, vp, i32, f32, vp, i32, vp, vp, i32, vp, vp, i32, vp]
         L.b200pose_transpose_planes.argtypes = [vp, vp, i32, i32, i32, vp, vp, i32, vp]
         L.b200pose_colsum.argtypes = [vp, i32, i32, i32, vp, i32, i32, vp, vp]
-        L.b200pose_fold_attention.argtypes = [vp, i32, vp, vp, vp, i32, i32, i32, vp, i32, vp, vp]
         L.b200pose_mse_sigmoid.argtypes = [vp, i32, vp, vp, i32, vp, vp, vp]
         L.b200pose_sigmoid_bwd.argtypes = [vp, vp, i32, vp, vp]
-        L.b200pose_adam_step.argtypes = [vp, vp, vp, vp, C.c_int64, f32, f32, f32, f32, f32, i32, vp]
         L.b200pose_gat_prepare_layer.argtypes = [vp, vp, i32, vp, vp, vp, i32, i32, i32, vp, vp, i32, vp, vp, i32, vp, vp, i32, vp, vp, i32, vp, vp]
         L.b200pose_gat_attn_bias_grad.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp, vp, vp, vp]
         L.b200pose_residual_bwd_add.argtypes = [vp, i32, vp, i32, i32, i32, i32, vp]

@@ -9,10 +9,6 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libb200pose.so')
-# the projection kernels again, with the superseded / bring-up variants compiled in (b200pose_linear impl 1, 2, 3, 6):
-# loaded only by tests/test_gpu_parity.py::test_linear_kernels, never by the package
-LIB_SELFTEST = os.path.join(HERE, 'libb200pose_selftest.so')
-SELFTEST_SOURCES = ['common.cu', 'gemm.cu']
 SOURCES = ['common.cu', 'graph.cu', 'gat.cu', 'cluster.cu', 'lift.cu', 'gemm.cu', 'pack_json.cu', 'train.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-Xcompiler', '-fvisibility=hidden']
@@ -26,7 +22,7 @@ def _nvcc():
 
 
 def needs_build():
-    if not os.path.exists(LIB) or not os.path.exists(LIB_SELFTEST):
+    if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, '..', 'include', 'b200pose.h')]
@@ -54,20 +50,6 @@ def build(force=False, verbose=True):
     subprocess.check_call(cmd)
     if verbose:
         print('built', LIB)
-    # self-test library (own object files: -DB200POSE_SELFTEST)
-    procs, objs = [], []
-    for src in SELFTEST_SOURCES:
-        obj = os.path.join(HERE, 'build', 'selftest_' + src.replace('.cu', '.o'))
-        objs.append(obj)
-        cmd = [_nvcc()] + NVCC_FLAGS + ['-DB200POSE_SELFTEST', '-c', os.path.join(CSRC, src), '-o', obj]
-        procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT)))
-    for src, p in procs:
-        out, _ = p.communicate()
-        if p.returncode != 0:
-            raise RuntimeError('nvcc failed on %s (self-test build):\n%s' % (src, out.decode()))
-    subprocess.check_call([_nvcc(), '-shared', '-o', LIB_SELFTEST] + objs + ['-gencode', 'arch=compute_100a,code=sm_100a'])
-    if verbose:
-        print('built', LIB_SELFTEST)
     return LIB
 
 

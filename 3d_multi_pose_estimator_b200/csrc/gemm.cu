@@ -5,14 +5,6 @@
 // attention dots of :57-58 folded in as extra output columns) and pose MLP (utils/mlp.py:8-28).
 // Plain bf16 or TF32 inputs miss the 1e-4 score / 0.5 mm joint tolerances (SURVEY.md 7-1), so every
 // fp32 operand is carried as two bf16 planes and each k-block issues three UMMA groups.
-//
-// Kernel anatomy (one 128 x bn output tile per CTA, 192 threads):
-//   warp 0 / lane 0 : TMA producer  - cp.async.bulk.tensor 2D, 128B-swizzled K-major tiles, mbarrier tx
-//   warp 1          : TMEM allocator; lane 0 issues tcgen05.mma (M=128, N=bn, K=16) and commits
-//   warps 2..5      : epilogue - tcgen05.ld 32 lanes x 32 columns, bias + LeakyReLU + scale, writes fp32
-//                     and/or re-split bf16 planes for the next GEMM
-// bn (multiple of 16, <= 256) and the pipeline depth are runtime values: the TMA box, the instruction
-// descriptor and the TMEM allocation all take them, so one kernel serves every layer shape.
 #include "common.cuh"
 #include <cuda.h>
 #include <cudaTypedefs.h>
@@ -97,174 +89,12 @@ __device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
     d |= (uint64_t)2 << 61;
     return d;
 }
-// kind::f16 instruction descriptor: D=f32, A=B=bf16, both K-major, M=128, N=bn
-__device__ __forceinline__ uint32_t make_idesc(int bn) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(bn >> 3) << 17) | ((uint32_t)(kBM >> 4) << 24);
-}
-
-struct GemmParams {
-    int M, N, num_kb, bn, stages;
-    const float* bias; float slope, out_scale;
-    float* out_f32; int ld_out;
-    __nv_bfloat16* out_hi; __nv_bfloat16* out_lo; int ld_planes;
-    // manual-fill (debug) variant only
-    const __nv_bfloat16* a_hi; const __nv_bfloat16* a_lo; int lda;
-    const __nv_bfloat16* w_hi; const __nv_bfloat16* w_lo; int ldw;
-};
-
-// 3 UMMA groups of one 64-wide k-block: hi*hi, lo*hi, hi*lo
-__device__ __forceinline__ void issue_kblock(uint32_t a_hi, uint32_t a_lo, uint32_t b_hi, uint32_t b_lo,
-                                             uint32_t tmem_d, uint32_t idesc, bool first)
-{
-#pragma unroll
-    for (int k4 = 0; k4 < kBK / kUmmaK; ++k4) {
-        const uint32_t off = k4 * kUmmaK * 2;                     // bytes inside the swizzle atom
-        const uint64_t dah = make_sw128_desc(a_hi + off), dal = make_sw128_desc(a_lo + off);
-        const uint64_t dbh = make_sw128_desc(b_hi + off), dbl = make_sw128_desc(b_lo + off);
-        umma_bf16(tmem_d, dah, dbh, idesc, (first && k4 == 0) ? 0u : 1u);
-        umma_bf16(tmem_d, dal, dbh, idesc, 1u);
-        umma_bf16(tmem_d, dah, dbl, idesc, 1u);
-    }
-}
-
-// epilogue of one tile: thread = one accumulator row; 32 columns per TMEM load
-__device__ __forceinline__ void epilogue_tile(const GemmParams& p, uint32_t tmem_base, int m0, int n0, int quarter, int lane)
-{
-    const int row = m0 + quarter * 32 + lane;
-    const bool row_ok = row < p.M;
-    for (int c0 = 0; c0 < p.bn; c0 += 32) {
-        uint32_t r[32];
-        tmem_ld_32x32(tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)c0, r);
-        const int ncols = min(32, p.bn - c0);                     // bn is a multiple of 16
-        float v[32];
-#pragma unroll
-        for (int i = 0; i < 32; ++i) {
-            const int col = n0 + c0 + i;
-            float x = 0.f;
-            if (i < ncols && col < p.N) {
-                x = __uint_as_float(r[i]) + (p.bias ? __ldg(p.bias + col) : 0.f);
-                x = leaky(x, p.slope) * p.out_scale;
-            }
-            v[i] = x;
-        }
-        if (!row_ok) continue;
-        if (p.out_f32) {
-            float* o = p.out_f32 + (size_t)row * p.ld_out + n0 + c0;
-            const bool vec_ok = ((p.ld_out & 3) == 0) && (((n0 + c0) & 3) == 0);
-#pragma unroll
-            for (int i = 0; i < 32; i += 4) {
-                if (i >= ncols) break;
-                if (vec_ok && n0 + c0 + i + 3 < p.N) {
-                    *reinterpret_cast<float4*>(o + i) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
-                } else {
-#pragma unroll
-                    for (int u = 0; u < 4; ++u)
-                        if (n0 + c0 + i + u < p.N) o[i + u] = v[i + u];
-                }
-            }
-        }
-        if (p.out_hi) {
-            uint32_t* oh = reinterpret_cast<uint32_t*>(p.out_hi + (size_t)row * p.ld_planes + n0 + c0);
-            uint32_t* ol = reinterpret_cast<uint32_t*>(p.out_lo + (size_t)row * p.ld_planes + n0 + c0);
-#pragma unroll
-            for (int i = 0; i < 32; i += 8) {
-                if (i < ncols && n0 + c0 + i + 7 < p.ld_planes) {           // ld_planes % 64 == 0, n0+c0 % 16 == 0
-                    uint32_t h[4], l[4];
-#pragma unroll
-                    for (int u = 0; u < 4; ++u) {
-                        __nv_bfloat16 h0, l0, h1, l1;
-                        split_bf16(v[i + 2 * u], h0, l0);
-                        split_bf16(v[i + 2 * u + 1], h1, l1);
-                        h[u] = pack_bf16x2(h0, h1);
-                        l[u] = pack_bf16x2(l0, l1);
-                    }
-                    *reinterpret_cast<uint4*>(oh + i / 2) = make_uint4(h[0], h[1], h[2], h[3]);
-                    *reinterpret_cast<uint4*>(ol + i / 2) = make_uint4(l[0], l[1], l[2], l[3]);
-                }
-            }
-        }
-    }
-}
 
 __device__ __forceinline__ uint32_t tmem_cols_for(int bn) {
     uint32_t c = 32;
     while ((int)c < bn) c <<= 1;
     return c;
 }
-
-#ifdef B200POSE_SELFTEST   // superseded / bring-up kernels: only in libb200pose_selftest.so (build.py --selftest), not in the product library
-// ------------------------------------------------------------------------------------------------
-// product kernel: TMA-fed, multi-stage
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kGemmThreads, 1) gemm_split_tc_kernel(
-    const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
-    const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo, const GemmParams p)
-{
-    extern __shared__ __align__(1024) uint8_t smem_dyn[];
-    __shared__ __align__(8) uint64_t bar_full[kMaxStages];
-    __shared__ __align__(8) uint64_t bar_empty[kMaxStages];
-    __shared__ __align__(8) uint64_t bar_acc;
-    __shared__ uint32_t tmem_slot;
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n0 = blockIdx.x * p.bn, m0 = blockIdx.y * kBM;
-    const uint32_t a_bytes = kBM * kBK * 2;                       // 16 KB per plane
-    const uint32_t b_bytes = (uint32_t)p.bn * kBK * 2;
-    const uint32_t stage_bytes = 2 * a_bytes + 2 * b_bytes;
-    const uint32_t tiles = (smem_u32(smem_dyn) + 1023u) & ~1023u;
-    const uint32_t ncols = tmem_cols_for(p.bn);
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < p.stages; ++s) { mbar_init(smem_u32(&bar_full[s]), 1); mbar_init(smem_u32(&bar_empty[s]), 1); }
-        mbar_init(smem_u32(&bar_acc), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) tmem_alloc(smem_u32(&tmem_slot), ncols);
-    tcgen05_fence_before();
-    __syncthreads();
-    tcgen05_fence_after();
-    const uint32_t tmem_base = tmem_slot;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            for (int kb = 0; kb < p.num_kb; ++kb) {
-                const int s = kb % p.stages;
-                const uint32_t ph = (uint32_t)(kb / p.stages) & 1u;
-                mbar_wait(smem_u32(&bar_empty[s]), ph ^ 1u);
-                const uint32_t full = smem_u32(&bar_full[s]);
-                mbar_expect_tx(full, stage_bytes);
-                const uint32_t base = tiles + (uint32_t)s * stage_bytes;
-                tma_load_2d(base, &map_a_hi, kb * kBK, m0, full);
-                tma_load_2d(base + a_bytes, &map_a_lo, kb * kBK, m0, full);
-                tma_load_2d(base + 2 * a_bytes, &map_w_hi, kb * kBK, n0, full);
-                tma_load_2d(base + 2 * a_bytes + b_bytes, &map_w_lo, kb * kBK, n0, full);
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            const uint32_t idesc = make_idesc(p.bn);
-            for (int kb = 0; kb < p.num_kb; ++kb) {
-                const int s = kb % p.stages;
-                const uint32_t ph = (uint32_t)(kb / p.stages) & 1u;
-                mbar_wait(smem_u32(&bar_full[s]), ph);
-                tcgen05_fence_after();
-                const uint32_t base = tiles + (uint32_t)s * stage_bytes;
-                issue_kblock(base, base + a_bytes, base + 2 * a_bytes, base + 2 * a_bytes + b_bytes, tmem_base, idesc, kb == 0);
-                umma_commit(smem_u32(&bar_empty[s]));             // frees the smem slot when these MMAs retire
-            }
-            umma_commit(smem_u32(&bar_acc));                      // accumulator complete
-        }
-    } else {
-        mbar_wait(smem_u32(&bar_acc), 0);
-        tcgen05_fence_after();
-        epilogue_tile(p, tmem_base, m0, n0, warp & 3, lane);
-    }
-    tcgen05_fence_before();
-    __syncthreads();
-    if (warp == 1) tmem_dealloc(tmem_base, ncols);
-}
-
-#endif  // B200POSE_SELFTEST
 
 // ------------------------------------------------------------------------------------------------
 // product kernel v2: persistent, double-buffered TMEM accumulators, TMA-store epilogue
@@ -293,11 +123,6 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
 }
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* map) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
-}
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
 }
 
 struct GemmParams2 {
@@ -723,349 +548,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_split_tc2_kernel(
     if (warp == 1) tmem_dealloc_n<NCTA>(tmem_base, ncols);
 }
 
-#ifdef B200POSE_SELFTEST   // superseded / bring-up kernels: only in libb200pose_selftest.so (build.py --selftest), not in the product library
-// ------------------------------------------------------------------------------------------------
-// Wide variant of the CTA-pair kernel for tall projections whose whole output width fits TMEM
-// (256 < N <= 512, i.e. 5..8 panels: the 400/420/320/336-wide GAT projections).
-//
-// The pair kernel above cuts such an N into two n-tiles and therefore streams the A tile through shared
-// memory twice per m-tile; measured with everything but the loads switched off (scripts/gemm_probe.py) the
-// L2->SM traffic alone costs 106 us of the 188 us of a 184320 x 400 x 400 projection. Here one tile spans the
-// full width: per k-block each CTA loads its 128 rows of A once and its share of BOTH halves of W, and the
-// leader issues two MMA groups per k-step - N=256 into TMEM columns [0,256) and N=bn-256 into [256,bn). The
-// accumulator is single-buffered (2 x 448 columns do not fit the 512 of TMEM), so the epilogue hands the two
-// column halves back separately: the MMAs of the next tile's lower half start while panels 4.. are still
-// being drained.
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kGemmThreads, 1) gemm_split_wide_kernel(
-    const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
-    const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,      // box: 128 W rows
-    const __grid_constant__ CUtensorMap map_w2_hi, const __grid_constant__ CUtensorMap map_w2_lo,    // box: (bn-256)/2 W rows
-    const __grid_constant__ CUtensorMap map_o_f32, const __grid_constant__ CUtensorMap map_o_hi,
-    const __grid_constant__ CUtensorMap map_o_lo, const GemmParams2 p)
-{
-    extern __shared__ __align__(1024) uint8_t smem_dyn[];
-    __shared__ __align__(8) uint64_t bar_full[kMaxStages];
-    __shared__ __align__(8) uint64_t bar_empty[kMaxStages];
-    __shared__ __align__(8) uint64_t bar_acc_full;
-    __shared__ __align__(8) uint64_t bar_acc_empty[2];          // [0]: columns < 256 drained, [1]: columns >= 256 drained
-    __shared__ uint32_t tmem_slot;
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const bool leader = rank == 0;
-    const int bn = p.stage_bn;                                   // full padded width, 320..512
-    const int bn_hi = bn - 256;                                  // width of the upper MMA group
-    const uint32_t a_bytes = kBM * kBK * 2;
-    const uint32_t blo_bytes = 128u * kBK * 2;                   // this CTA's 128 W rows of the lower group, per plane
-    const uint32_t bhi_bytes = (uint32_t)(bn_hi / 2) * kBK * 2;  // and its share of the upper group
-    const uint32_t stage_bytes = 2 * a_bytes + 2 * blo_bytes + 2 * bhi_bytes;
-    const uint32_t tiles_base = (smem_u32(smem_dyn) + 1023u) & ~1023u;
-    const uint32_t staging_base = tiles_base + (uint32_t)p.stages * stage_bytes;
-    const int workers = gridDim.x / 2, worker = blockIdx.x / 2;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < p.stages; ++s) { mbar_init(smem_u32(&bar_full[s]), 1); mbar_init(smem_u32(&bar_empty[s]), 1); }
-        mbar_init(smem_u32(&bar_acc_full), 1);
-        mbar_init(smem_u32(&bar_acc_empty[0]), 8);
-        mbar_init(smem_u32(&bar_acc_empty[1]), 8);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        prefetch_tmap(&map_a_hi); prefetch_tmap(&map_a_lo); prefetch_tmap(&map_w_hi); prefetch_tmap(&map_w_lo);
-        prefetch_tmap(&map_w2_hi); prefetch_tmap(&map_w2_lo);
-        if (p.has_f32) prefetch_tmap(&map_o_f32);
-        if (p.has_planes) { prefetch_tmap(&map_o_hi); prefetch_tmap(&map_o_lo); }
-    }
-    if (warp == 1) tmem_alloc_n<2>(smem_u32(&tmem_slot), 512);
-    tcgen05_fence_before();
-    cluster_sync_all();
-    tcgen05_fence_after();
-    const uint32_t tmem_base = tmem_slot;
-
-    if (warp == 0) {
-        // ================= TMA producer =================
-        if (lane == 0) {
-            int it = 0;
-            const uint32_t tx = 2 * stage_bytes;                 // both CTAs' bytes land on the leader's barrier
-            for (int mb = worker; mb < p.tiles_m; mb += workers) {
-                const int m_cta = mb * 2 * kBM + (int)rank * kBM;
-                for (int kb = 0; kb < p.num_kb; ++kb, ++it) {
-                    const int s = it % p.stages;
-                    const uint32_t ph = (uint32_t)(it / p.stages) & 1u;
-                    mbar_wait(smem_u32(&bar_empty[s]), ph ^ 1u);
-                    const uint32_t full = smem_u32(&bar_full[s]);
-                    const uint32_t base = tiles_base + (uint32_t)s * stage_bytes;
-                    if (leader) mbar_expect_tx(full, tx);
-                    const uint32_t full0 = mapa_shared(full, 0);
-                    tma_load_2d_pair(base, &map_a_hi, kb * kBK, m_cta, full0);
-                    tma_load_2d_pair(base + a_bytes, &map_a_lo, kb * kBK, m_cta, full0);
-                    const uint32_t b0 = base + 2 * a_bytes;
-                    tma_load_2d_pair(b0, &map_w_hi, kb * kBK, (int)rank * 128, full0);
-                    tma_load_2d_pair(b0 + blo_bytes, &map_w_lo, kb * kBK, (int)rank * 128, full0);
-                    tma_load_2d_pair(b0 + 2 * blo_bytes, &map_w2_hi, kb * kBK, 256 + (int)rank * (bn_hi / 2), full0);
-                    tma_load_2d_pair(b0 + 2 * blo_bytes + bhi_bytes, &map_w2_lo, kb * kBK, 256 + (int)rank * (bn_hi / 2), full0);
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ================= MMA issuer (leader CTA) =================
-        if (lane == 0 && leader) {
-            const uint32_t idesc_lo = make_idesc_n<2>(256), idesc_hi = make_idesc_n<2>(bn_hi);
-            int it = 0, i = 0;
-            for (int mb = worker; mb < p.tiles_m; mb += workers, ++i) {
-                const uint32_t pe = ((uint32_t)i & 1u) ^ 1u;     // phase i-1 of the drained barriers (fresh barrier: passes)
-                for (int kb = 0; kb < p.num_kb; ++kb, ++it) {
-                    const int s = it % p.stages;
-                    const uint32_t ph = (uint32_t)(it / p.stages) & 1u;
-                    mbar_wait(smem_u32(&bar_full[s]), ph);
-                    tcgen05_fence_after();
-                    const uint32_t base = tiles_base + (uint32_t)s * stage_bytes;
-                    const uint32_t sa_hi = base, sa_lo = base + a_bytes, b0 = base + 2 * a_bytes;
-                    if (kb == 0) { mbar_wait(smem_u32(&bar_acc_empty[0]), pe); tcgen05_fence_after(); }
-#pragma unroll
-                    for (int k4 = 0; k4 < kBK / kUmmaK; ++k4) {
-                        const uint32_t off = k4 * kUmmaK * 2;
-                        const uint64_t dah = make_sw128_desc(sa_hi + off), dal = make_sw128_desc(sa_lo + off);
-                        const uint64_t dbh = make_sw128_desc(b0 + off), dbl = make_sw128_desc(b0 + blo_bytes + off);
-                        const uint32_t first = (kb == 0 && k4 == 0) ? 0u : 1u;
-                        umma_bf16_pair(tmem_base, dah, dbh, idesc_lo, first);
-                        umma_bf16_pair(tmem_base, dal, dbh, idesc_lo, 1u);
-                        umma_bf16_pair(tmem_base, dah, dbl, idesc_lo, 1u);
-                    }
-                    if (kb == 0) { mbar_wait(smem_u32(&bar_acc_empty[1]), pe); tcgen05_fence_after(); }
-#pragma unroll
-                    for (int k4 = 0; k4 < kBK / kUmmaK; ++k4) {
-                        const uint32_t off = k4 * kUmmaK * 2;
-                        const uint64_t dah = make_sw128_desc(sa_hi + off), dal = make_sw128_desc(sa_lo + off);
-                        const uint64_t dbh = make_sw128_desc(b0 + 2 * blo_bytes + off), dbl = make_sw128_desc(b0 + 2 * blo_bytes + bhi_bytes + off);
-                        const uint32_t first = (kb == 0 && k4 == 0) ? 0u : 1u;
-                        umma_bf16_pair(tmem_base + 256u, dah, dbh, idesc_hi, first);
-                        umma_bf16_pair(tmem_base + 256u, dal, dbh, idesc_hi, 1u);
-                        umma_bf16_pair(tmem_base + 256u, dah, dbl, idesc_hi, 1u);
-                    }
-                    umma_commit_pair(smem_u32(&bar_empty[s]));
-                }
-                umma_commit_pair(smem_u32(&bar_acc_full));
-            }
-        }
-    } else {
-        // ================= epilogue =================
-        const int q = warp & 3;
-        const uint32_t stage_f32 = staging_base + (uint32_t)(warp - 2) * (uint32_t)((p.has_f32 ? 8192 : 0) + (p.has_planes ? 8192 : 0));
-        const uint32_t stage_hi = stage_f32 + (p.has_f32 ? 8192u : 0u);
-        const uint32_t stage_lo = stage_hi + 4096u;
-        const uint32_t sw = (uint32_t)(lane & 7);
-        const uint32_t row_off = (uint32_t)lane * 128u;
-        const uint32_t tmem_t = tmem_base + ((uint32_t)(q * 32) << 16);
-        const int npanels = bn / 64;
-        bool stores_pending = false;
-        const bool slope_le1 = p.slope >= 0.f && p.slope <= 1.f;
-        int i = 0;
-        for (int mb = worker; mb < p.tiles_m; mb += workers, ++i) {
-            mbar_wait(smem_u32(&bar_acc_full), (uint32_t)i & 1u);
-            tcgen05_fence_after();
-            for (int j = 0; j < npanels; ++j) {
-                const int col0 = 64 * j;
-                uint32_t r0[32], r1[32];
-                tmem_ld_32x32(tmem_t + (uint32_t)(64 * j), r0);
-                tmem_ld_32x32(tmem_t + (uint32_t)(64 * j + 32), r1);
-                if (j == 3 || j == npanels - 1) {                 // a column half is drained: hand it back to the MMA warp
-                    tcgen05_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive_cluster(mapa_shared(smem_u32(&bar_acc_empty[j == 3 ? 0 : 1]), 0));
-                }
-                float b0 = 0.f, b1 = 0.f;
-                if (p.bias) {
-                    if (col0 + lane < p.N) b0 = __ldg(p.bias + col0 + lane);
-                    if (col0 + 32 + lane < p.N) b1 = __ldg(p.bias + col0 + 32 + lane);
-                }
-                float v[64];
-                if (slope_le1) {
-#pragma unroll
-                    for (int c = 0; c < 32; ++c) {
-                        const float bb0 = __shfl_sync(0xffffffffu, b0, c), bb1 = __shfl_sync(0xffffffffu, b1, c);
-                        v[c] = (col0 + c < p.N) ? leaky_le1(__uint_as_float(r0[c]) + bb0, p.slope) * p.out_scale : 0.f;
-                        v[32 + c] = (col0 + 32 + c < p.N) ? leaky_le1(__uint_as_float(r1[c]) + bb1, p.slope) * p.out_scale : 0.f;
-                    }
-                } else {
-#pragma unroll
-                    for (int c = 0; c < 32; ++c) {
-                        const float bb0 = __shfl_sync(0xffffffffu, b0, c), bb1 = __shfl_sync(0xffffffffu, b1, c);
-                        v[c] = (col0 + c < p.N) ? leaky(__uint_as_float(r0[c]) + bb0, p.slope) * p.out_scale : 0.f;
-                        v[32 + c] = (col0 + 32 + c < p.N) ? leaky(__uint_as_float(r1[c]) + bb1, p.slope) * p.out_scale : 0.f;
-                    }
-                }
-                if (stores_pending) {
-                    if (lane == 0) bulk_wait_read0();
-                    __syncwarp();
-                }
-                if (p.has_f32) {
-#pragma unroll
-                    for (int half = 0; half < 2; ++half)
-#pragma unroll
-                        for (int c = 0; c < 8; ++c) {
-                            const uint32_t addr = stage_f32 + (uint32_t)half * 4096u + row_off + (((uint32_t)c ^ sw) << 4);
-                            asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(v[half * 32 + 4 * c]),
-                                         "f"(v[half * 32 + 4 * c + 1]), "f"(v[half * 32 + 4 * c + 2]), "f"(v[half * 32 + 4 * c + 3]) : "memory");
-                        }
-                }
-                if (p.has_planes) {
-#pragma unroll
-                    for (int c = 0; c < 8; ++c) {
-                        uint32_t h[4], l[4];
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) split_pack2(v[8 * c + 2 * u], v[8 * c + 2 * u + 1], h[u], l[u]);
-                        const uint32_t off = row_off + (((uint32_t)c ^ sw) << 4);
-                        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stage_hi + off), "r"(h[0]), "r"(h[1]), "r"(h[2]), "r"(h[3]) : "memory");
-                        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(stage_lo + off), "r"(l[0]), "r"(l[1]), "r"(l[2]), "r"(l[3]) : "memory");
-                    }
-                }
-                fence_async_smem();
-                __syncwarp();
-                if (lane == 0) {
-                    const int row0 = mb * 2 * kBM + (int)rank * kBM + q * 32;
-                    if (row0 < p.M && !(p.dbg & 1)) {
-                        if (p.has_f32) {
-                            if (col0 < p.N) tma_store_2d(&map_o_f32, stage_f32, col0, row0);
-                            if (col0 + 32 < p.N) tma_store_2d(&map_o_f32, stage_f32 + 4096u, col0 + 32, row0);
-                        }
-                        if (p.has_planes) {
-                            tma_store_2d(&map_o_hi, stage_hi, col0, row0);
-                            tma_store_2d(&map_o_lo, stage_lo, col0, row0);
-                        }
-                    }
-                    bulk_commit();
-                }
-                stores_pending = true;
-            }
-        }
-        if (lane == 0) bulk_wait0();
-    }
-    tcgen05_fence_before();
-    cluster_sync_all();
-    if (warp == 1) tmem_dealloc_n<2>(tmem_base, 512);
-}
-
-#endif  // B200POSE_SELFTEST
-
-#ifdef B200POSE_SELFTEST   // superseded / bring-up kernels: only in libb200pose_selftest.so (build.py --selftest), not in the product library
-// ------------------------------------------------------------------------------------------------
-// debug kernel: identical MMA + epilogue, but the tiles are written by ordinary stores (no TMA,
-// single stage). Used by the kernel self-test to separate tensor-map bugs from descriptor bugs.
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void fill_tile_sw128(uint8_t* tile, const __nv_bfloat16* g, int ld, int row0, int rows_valid,
-                                                int rows_tile, int k0, int tid, int nthreads)
-{
-    // 16-byte chunks: chunk c of row r lands at r*128 + ((c ^ (r & 7)) << 4)
-    for (int i = tid; i < rows_tile * 8; i += nthreads) {
-        const int r = i >> 3, c = i & 7;
-        uint4 v = make_uint4(0, 0, 0, 0);
-        if (r < rows_valid) v = *reinterpret_cast<const uint4*>(g + (size_t)(row0 + r) * ld + k0 + c * 8);
-        *reinterpret_cast<uint4*>(tile + r * 128 + ((c ^ (r & 7)) << 4)) = v;
-    }
-}
-
-__global__ void __launch_bounds__(kGemmThreads, 1) gemm_split_tc_manual_kernel(const GemmParams p)
-{
-    extern __shared__ __align__(1024) uint8_t smem_dyn[];
-    __shared__ __align__(8) uint64_t bar_mma;
-    __shared__ uint32_t tmem_slot;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n0 = blockIdx.x * p.bn, m0 = blockIdx.y * kBM;
-    const uint32_t a_bytes = kBM * kBK * 2, b_bytes = (uint32_t)p.bn * kBK * 2;
-    uint8_t* tiles_g = smem_dyn + (((smem_u32(smem_dyn) + 1023u) & ~1023u) - smem_u32(smem_dyn));
-    const uint32_t tiles = smem_u32(tiles_g);
-    const uint32_t ncols = tmem_cols_for(p.bn);
-    if (threadIdx.x == 0) {
-        mbar_init(smem_u32(&bar_mma), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) tmem_alloc(smem_u32(&tmem_slot), ncols);
-    tcgen05_fence_before();
-    __syncthreads();
-    tcgen05_fence_after();
-    const uint32_t tmem_base = tmem_slot;
-    const uint32_t idesc = make_idesc(p.bn);
-    for (int kb = 0; kb < p.num_kb; ++kb) {
-        fill_tile_sw128(tiles_g, p.a_hi, p.lda, m0, max(0, min(kBM, p.M - m0)), kBM, kb * kBK, threadIdx.x, kGemmThreads);
-        fill_tile_sw128(tiles_g + a_bytes, p.a_lo, p.lda, m0, max(0, min(kBM, p.M - m0)), kBM, kb * kBK, threadIdx.x, kGemmThreads);
-        fill_tile_sw128(tiles_g + 2 * a_bytes, p.w_hi, p.ldw, n0, max(0, min(p.bn, p.N - n0)), p.bn, kb * kBK, threadIdx.x, kGemmThreads);
-        fill_tile_sw128(tiles_g + 2 * a_bytes + b_bytes, p.w_lo, p.ldw, n0, max(0, min(p.bn, p.N - n0)), p.bn, kb * kBK, threadIdx.x, kGemmThreads);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");       // generic-proxy writes -> async proxy (UMMA)
-        __syncthreads();
-        if (warp == 1 && lane == 0) {
-            tcgen05_fence_after();
-            issue_kblock(tiles, tiles + a_bytes, tiles + 2 * a_bytes, tiles + 2 * a_bytes + b_bytes, tmem_base, idesc, kb == 0);
-            umma_commit(smem_u32(&bar_mma));
-        }
-        mbar_wait(smem_u32(&bar_mma), (uint32_t)kb & 1u);                    // tiles may be overwritten now
-        __syncthreads();
-    }
-    tcgen05_fence_after();
-    if (warp >= 2) epilogue_tile(p, tmem_base, m0, n0, warp & 3, lane);
-    tcgen05_fence_before();
-    __syncthreads();
-    if (warp == 1) tmem_dealloc(tmem_base, ncols);
-}
-
-// ------------------------------------------------------------------------------------------------
-// fp32 SIMT kernel on the same planes (kernel self-test reference; not on the product path)
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) gemm_split_simt_kernel(const GemmParams p, int K)
-{
-    __shared__ float As[64][17];
-    __shared__ float Ws[64][17];
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const int m0 = blockIdx.y * 64, n0 = blockIdx.x * 64;
-    float acc[4][4] = {};
-    for (int k0 = 0; k0 < K; k0 += 16) {
-        for (int i = threadIdx.x; i < 64 * 16; i += 256) {
-            const int r = i >> 4, c = i & 15;
-            float a = 0.f, w = 0.f;
-            if (m0 + r < p.M && k0 + c < K) {
-                const size_t o = (size_t)(m0 + r) * p.lda + k0 + c;
-                a = __bfloat162float(p.a_hi[o]) + __bfloat162float(p.a_lo[o]);
-            }
-            if (n0 + r < p.N && k0 + c < K) {
-                const size_t o = (size_t)(n0 + r) * p.ldw + k0 + c;
-                w = __bfloat162float(p.w_hi[o]) + __bfloat162float(p.w_lo[o]);
-            }
-            As[r][c] = a; Ws[r][c] = w;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int k = 0; k < 16; ++k) {
-            float a[4], w[4];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) { a[i] = As[ty * 4 + i][k]; w[i] = Ws[tx * 4 + i][k]; }
-#pragma unroll
-            for (int i = 0; i < 4; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(a[i], w[j], acc[i][j]);
-        }
-        __syncthreads();
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int row = m0 + ty * 4 + i;
-        if (row >= p.M) continue;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const int col = n0 + tx * 4 + j;
-            float x = 0.f;
-            if (col < p.N) x = leaky(acc[i][j] + (p.bias ? p.bias[col] : 0.f), p.slope) * p.out_scale;
-            if (p.out_f32 && col < p.N) p.out_f32[(size_t)row * p.ld_out + col] = x;
-            if (p.out_hi && col < p.ld_planes) {
-                __nv_bfloat16 h, l;
-                split_bf16(x, h, l);
-                p.out_hi[(size_t)row * p.ld_planes + col] = h;
-                p.out_lo[(size_t)row * p.ld_planes + col] = l;
-            }
-        }
-    }
-}
-
-#endif  // B200POSE_SELFTEST
-
 // ------------------------------------------------------------------------------------------------
 // Small-M kernel (m <= 8 rows: the pose MLP of a single frame). With a handful of rows the projection is a
 // weight-streaming problem - the MLP holds 116 MB of hi/lo weights - and the tensor-core kernel would read them
@@ -1303,13 +785,6 @@ static int num_sms() {
     return n;
 }
 
-static int choose_bn(int n) {
-    const int tiles = ceil_div(n, 256);
-    int bn = ceil_div(ceil_div(n, tiles), 16) * 16;
-    if (bn < 16) bn = 16;
-    return bn;
-}
-
 }  // namespace b200pose
 
 using namespace b200pose;
@@ -1323,6 +798,8 @@ static int linear_impl(const uint16_t* a_hi, const uint16_t* a_lo, int32_t lda,
                        float* out_f32, int32_t ld_out, uint16_t* out_hi, uint16_t* out_lo, int32_t ld_planes,
                        int32_t impl, void* stream, const FuseArgs* fuse = nullptr)
 {
+    B2_CHECK_ARG(impl == 0 || impl == 4 || impl == 5 || impl == 7, "linear: impl must be 0 (dispatch), 4 (persistent, single CTAs), "
+                 "5 (persistent, CTA pairs) or 7 (few-row kernels when m <= 16)");
     B2_CHECK_ARG(a_hi && a_lo && w_hi && w_lo, "linear: null operand");
     if (fuse) {
         B2_CHECK_ARG(impl == 0 && !m_dev, "linear_fused2: impl must be 0");
@@ -1344,55 +821,13 @@ static int linear_impl(const uint16_t* a_hi, const uint16_t* a_lo, int32_t lda,
                  "linear: operands must be 16-byte aligned");
     if (m == 0) return B200POSE_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    GemmParams p;
-    p.M = m; p.N = n; p.num_kb = kpad / kBK; p.bias = bias; p.slope = slope; p.out_scale = out_scale;
-    p.out_f32 = out_f32; p.ld_out = ld_out;
-    p.out_hi = reinterpret_cast<__nv_bfloat16*>(out_hi); p.out_lo = reinterpret_cast<__nv_bfloat16*>(out_lo); p.ld_planes = ld_planes;
-    p.a_hi = reinterpret_cast<const __nv_bfloat16*>(a_hi); p.a_lo = reinterpret_cast<const __nv_bfloat16*>(a_lo); p.lda = lda;
-    p.w_hi = reinterpret_cast<const __nv_bfloat16*>(w_hi); p.w_lo = reinterpret_cast<const __nv_bfloat16*>(w_lo); p.ldw = ldw;
-    p.bn = choose_bn(n);
-    p.stages = 1;
-#ifdef B200POSE_SELFTEST
-    if (impl == 1) {
-        const int cols = (out_hi && ld_planes > n) ? ld_planes : n;     // also zero the K padding of the planes
-        dim3 grid(ceil_div(cols, 64), ceil_div(m, 64));
-        gemm_split_simt_kernel<<<grid, 256, 0, st>>>(p, k);
-        B2_CHECK_LAUNCH();
-        return B200POSE_OK;
-    }
-    const size_t stage_bytes = 2 * (size_t)kBM * kBK * 2 + 2 * (size_t)p.bn * kBK * 2;
-    dim3 grid(ceil_div(n, p.bn), ceil_div(m, kBM));
-    if (impl == 2) {
-        const size_t smem = stage_bytes + 1024;
-        B2_CHECK_CUDA(cudaFuncSetAttribute(gemm_split_tc_manual_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        gemm_split_tc_manual_kernel<<<grid, kGemmThreads, smem, st>>>(p);
-        B2_CHECK_LAUNCH();
-        return B200POSE_OK;
-    }
-    if (impl == 3) {                       // v1 non-persistent kernel, kept for A/B measurements during bring-up
-        int stages = (int)((220 * 1024 - 1024) / stage_bytes);
-        if (stages > kMaxStages) stages = kMaxStages;
-        if (stages > p.num_kb) stages = p.num_kb;
-        if (stages < 1) stages = 1;
-        p.stages = stages;
-        const size_t smem = (size_t)stages * stage_bytes + 1024;
-        CUtensorMap ma_hi, ma_lo, mw_hi, mw_lo;
-        int rc;
-        if ((rc = make_map(&ma_hi, a_hi, m, kpad, lda, kBM))) return rc;
-        if ((rc = make_map(&ma_lo, a_lo, m, kpad, lda, kBM))) return rc;
-        if ((rc = make_map(&mw_hi, w_hi, n, kpad, ldw, p.bn))) return rc;
-        if ((rc = make_map(&mw_lo, w_lo, n, kpad, ldw, p.bn))) return rc;
-        B2_CHECK_CUDA(cudaFuncSetAttribute(gemm_split_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        gemm_split_tc_kernel<<<grid, kGemmThreads, smem, st>>>(ma_hi, ma_lo, mw_hi, mw_lo, p);
-        B2_CHECK_LAUNCH();
-        return B200POSE_OK;
-    }
-#else
-    if (impl == 1 || impl == 2 || impl == 3 || impl == 6) {
-        set_error("linear: impl 1/2/3/6 are bring-up kernels of the self-test build (libb200pose_selftest.so), not part of the product library");
-        return B200POSE_E_UNSUPPORTED;
-    }
-#endif
+    // the few-row kernels take the planes as bf16 pointers
+    const __nv_bfloat16* ah = reinterpret_cast<const __nv_bfloat16*>(a_hi);
+    const __nv_bfloat16* al = reinterpret_cast<const __nv_bfloat16*>(a_lo);
+    const __nv_bfloat16* wh = reinterpret_cast<const __nv_bfloat16*>(w_hi);
+    const __nv_bfloat16* wl = reinterpret_cast<const __nv_bfloat16*>(w_lo);
+    __nv_bfloat16* oh = reinterpret_cast<__nv_bfloat16*>(out_hi);
+    __nv_bfloat16* ol = reinterpret_cast<__nv_bfloat16*>(out_lo);
     if (!m_dev && !fuse && (impl == 0 || impl == 7) && m <= 8 && kpad <= 4096 && lda % 8 == 0 && ldw % 8 == 0) {
         // weight stream with A in registers: k split over the CTA's lanes, blocks of 32 / MMAX columns
         const int warps = ceil_div(kpad, 256);
@@ -1401,8 +836,8 @@ static int linear_impl(const uint16_t* a_hi, const uint16_t* a_lo, int32_t lda,
         auto launch_stream = [&](auto kern, int c_per_block) -> int {
             int ctas = ceil_div(cols, c_per_block);
             if (ctas > num_sms() * per_sm) ctas = num_sms() * per_sm;
-            kern<<<ctas, warps * 32, 0, st>>>(p.a_hi, p.a_lo, lda, p.w_hi, p.w_lo, ldw, bias, m, n, kpad, slope, out_scale,
-                                              out_f32, ld_out, p.out_hi, p.out_lo, ld_planes);
+            kern<<<ctas, warps * 32, 0, st>>>(ah, al, lda, wh, wl, ldw, bias, m, n, kpad, slope, out_scale,
+                                              out_f32, ld_out, oh, ol, ld_planes);
             B2_CHECK_LAUNCH();
             return B200POSE_OK;
         };
@@ -1417,22 +852,20 @@ static int linear_impl(const uint16_t* a_hi, const uint16_t* a_lo, int32_t lda,
         if (ctas > cap) ctas = cap;
         auto launch_small = [&](auto kern) -> int {
             B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            kern<<<ctas, kSmallWarps * 32, smem, st>>>(p.a_hi, p.a_lo, lda, p.w_hi, p.w_lo, ldw, bias, m, n, kpad, slope, out_scale,
-                                                       out_f32, ld_out, p.out_hi, p.out_lo, ld_planes);
+            kern<<<ctas, kSmallWarps * 32, smem, st>>>(ah, al, lda, wh, wl, ldw, bias, m, n, kpad, slope, out_scale,
+                                                       out_f32, ld_out, oh, ol, ld_planes);
             B2_CHECK_LAUNCH();
             return B200POSE_OK;
         };
         return m <= 8 ? launch_small(gemm_small_m_kernel<8>) : launch_small(gemm_small_m_kernel<16>);
     }
-    B2_CHECK_ARG(impl == 0 || impl == 4 || impl == 5 || impl == 6 || impl == 7, "linear: impl must be 0 (auto), 1 (simt self-test), 2 (manual-fill "
-                 "self-test), 3 (v1), 4 (persistent, single CTA), 5 (CTA pairs), 6 (wide CTA pairs) or 7 (small-m kernel when m <= 16)");
     // ---- persistent kernel ----
     if (out_f32) B2_CHECK_ARG(ld_out % 4 == 0 && ((uintptr_t)out_f32 % 16 == 0), "linear: out_f32 needs ld_out %% 4 == 0 and 16-byte alignment (TMA store)");
     if (out_hi) B2_CHECK_ARG(((uintptr_t)out_hi % 16 == 0) && ((uintptr_t)out_lo % 16 == 0), "linear: output planes must be 16-byte aligned");
     // CTA pairs (cta_group::2, 256-row tiles) as soon as there is more than one pair tile of rows: per flop a pair pulls
     // 1.5x fewer bytes through the L2->SM fabric, which bounds both the tall GAT projections and the MLP (every m-tile
     // re-reads the whole weight matrix from L2)
-    const int ncta = (impl == 5 || impl == 6) ? 2 : (impl == 4) ? 1 : (m > 4 * kBM ? 2 : 1);
+    const int ncta = (impl == 5) ? 2 : (impl == 4) ? 1 : (m > 4 * kBM ? 2 : 1);
     GemmParams2 q;
     q.M = m; q.N = n; q.num_kb = kpad / kBK; q.k_last = ceil_div(k - (kpad / kBK - 1) * kBK, kUmmaK); q.bias = bias; q.slope = slope; q.out_scale = out_scale;
     q.has_f32 = out_f32 ? 1 : 0; q.has_planes = out_hi ? 1 : 0; q.dbg = g_debug_flags; q.m_dev = m_dev;
@@ -1453,38 +886,6 @@ static int linear_impl(const uint16_t* a_hi, const uint16_t* a_lo, int32_t lda,
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-#ifdef B200POSE_SELFTEST
-    // ---- wide pair kernel: tall projections whose whole width fits TMEM (5..8 panels): A streamed once per m-tile ----
-    // Measured on B200 (GAT projections, 184320 rows): 1.43 ms per step against 1.20 ms for the two-n-tile pair kernel -
-    // the 88 KB stages leave room for only two of them and the single-buffered accumulator exposes the epilogue, which
-    // costs more than streaming A twice. Kept selectable (impl 6) for A/B runs; not on the product path.
-    const bool wide = impl == 6 && q.panels_total > 4 && q.panels_total <= 8;
-    if (wide) {
-        q.tiles_m = ceil_div(m, 2 * kBM);
-        q.tiles_n = 1;
-        q.group_n = 1;
-        q.stage_bn = 64 * q.panels_total;
-        const int bn_hi = q.stage_bn - 256;
-        const size_t stage_w = 2 * (size_t)kBM * kBK * 2 + 2 * (size_t)128 * kBK * 2 + 2 * (size_t)(bn_hi / 2) * kBK * 2;
-        int stages = (int)((227 * 1024 - 2048 - staging) / stage_w);
-        if (stages > kMaxStages) stages = kMaxStages;
-        if (stages >= 2) {
-            q.stages = stages;
-            const size_t smem = (size_t)stages * stage_w + staging + 1024;
-            if ((rc = make_map(&mw_hi, w_hi, n, kpad, ldw, 128))) return rc;
-            if ((rc = make_map(&mw_lo, w_lo, n, kpad, ldw, 128))) return rc;
-            if ((rc = make_map(&mw2_hi, w_hi, n, kpad, ldw, bn_hi / 2))) return rc;
-            if ((rc = make_map(&mw2_lo, w_lo, n, kpad, ldw, bn_hi / 2))) return rc;
-            const int workers = q.tiles_m < num_sms() / 2 ? q.tiles_m : num_sms() / 2;
-            B2_CHECK_CUDA(cudaFuncSetAttribute(gemm_split_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3(2 * workers); cfg.blockDim = dim3(kGemmThreads); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-            cfg.attrs = attr; cfg.numAttrs = 1;
-            B2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, gemm_split_wide_kernel, ma_hi, ma_lo, mw_hi, mw_lo, mw2_hi, mw2_lo, mo_f32, mo_hi, mo_lo, q));
-            return B200POSE_OK;
-        }
-    }
-#endif
     q.tiles_n = ceil_div(q.panels_total, 4);
     q.tiles_m = ceil_div(m, kBM * ncta);
     // a handful of m-tiles (single-frame calls: ~180 graph nodes): one 64-column panel per tile, so that the k-loops of

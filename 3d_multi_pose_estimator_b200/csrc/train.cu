@@ -223,36 +223,13 @@ __global__ void __launch_bounds__(1024) colsum_kernel(const float* __restrict__ 
     }
 }
 
-// [W2 ; attn_l-folded rows ; attn_r-folded rows]: a1[n, h] = sum_d ft2[n, h, d] attn_l[h, d] = h2[n, :] . (sum_d attn_l[h, d] W2[hD + d, :]) + ...
-// (gat2.py:55-58), so fc2 yields [ft2 | a1 | a2] in one GEMM. fp64 accumulation as the inference path's host-side fold.
-__global__ void __launch_bounds__(256) fold_attention_kernel(const float* __restrict__ W2, int ld_w2, const float* __restrict__ b2,
-                                                            const float* __restrict__ attn_l, const float* __restrict__ attn_r,
-                                                            int H, int D, int din, float* __restrict__ W2e, int ld_w2e, float* __restrict__ b2e)
-{
-    const int HD = H * D;
-    const int total_rows = HD + 2 * H;
-    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const int cols = din + 1;                                  // column `din` = the bias
-    if (idx >= (long long)total_rows * cols) return;
-    const int r = (int)(idx / cols), c = (int)(idx % cols);
-    double v;
-    if (r < HD) {
-        v = c < din ? W2[(size_t)r * ld_w2 + c] : b2[r];
-    } else {
-        const int h = (r - HD) % H;
-        const float* a = (r - HD) < H ? attn_l : attn_r;
-        v = 0.0;
-        for (int d = 0; d < D; ++d)
-            v += (double)a[h * D + d] * (double)(c < din ? W2[(size_t)(h * D + d) * ld_w2 + c] : b2[h * D + d]);
-    }
-    if (c < din) W2e[(size_t)r * ld_w2e + c] = (float)v; else b2e[r] = (float)v;
-}
-
 // Every operand plane of one layer from its fp32 parameters, in one launch (after each optimiser step): W1 -> planes and
 // transposed planes; [W2 ; attention folds] -> planes (+ the folded bias); W2 -> transposed planes. One CTA per 32x32 tile of
 // two stacked index spaces (rows_a rows of W1, then rows_b rows of [W2 ; folds]); the transposed planes go through a
 // shared-memory tile so that both layouts are written with coalesced stores. Paddings are written as zeros so the planes can
 // be consumed as K padding.
+// The folds: a1[n, h] = sum_d ft2[n, h, d] attn_l[h, d] = h2[n, :] . (sum_d attn_l[h, d] W2[hD + d, :]) + ... (gat2.py:55-58),
+// so fc2 yields [ft2 | a1 | a2] in one GEMM. fp64 accumulation as the inference path's host-side fold.
 __device__ __forceinline__ float fold_row_value(const float* __restrict__ W2, int ld_w, const float* __restrict__ attn_l,
                                                 const float* __restrict__ attn_r, int H, int D, int HD, int r, int c)
 {
@@ -393,25 +370,6 @@ __global__ void __launch_bounds__(256) sigmoid_bwd_kernel(const float* __restric
     if (i < n) { const float p = scores[i]; dlogit[i] = dscores[i] * p * (1.f - p); }
 }
 
-// torch.optim.Adam, single-tensor form (amsgrad off): exp_avg.lerp_(g, 1 - b1); exp_avg_sq = b2 v + (1 - b2) g g;
-// denom = sqrt(v) / sqrt(1 - b2^t) + eps; theta -= lr / (1 - b1^t) * m / denom
-__global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ theta, const float* __restrict__ grad, float* __restrict__ m,
-                                                  float* __restrict__ v, long long n, float b1, float b2, float eps, float wd,
-                                                  float step_size, float bc2_sqrt)
-{
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    float g = grad[i];
-    const float th = theta[i];
-    if (wd != 0.f) g = fmaf(wd, th, g);
-    float mi = m[i], vi = v[i];
-    mi = mi + (g - mi) * (1.f - b1);
-    vi = vi * b2 + (1.f - b2) * g * g;
-    m[i] = mi; v[i] = vi;
-    const float denom = sqrtf(vi) / bc2_sqrt + eps;
-    theta[i] = th - step_size * (mi / denom);
-}
-
 // Adam with the step count on the device (so a whole optimisation step can be replayed as a CUDA graph): one thread advances
 // the counter and writes step_size = lr / (1 - b1^t) and sqrt(1 - b2^t) for the element kernel that follows
 __global__ void adam_scalars_kernel(int* __restrict__ step, float lr, float b1, float b2, float* __restrict__ scal)
@@ -422,7 +380,9 @@ __global__ void adam_scalars_kernel(int* __restrict__ step, float lr, float b1, 
     scal[1] = (float)sqrt(1.0 - pow((double)b2, (double)t));
 }
 
-// one element of the device-step Adam; shared by adam_dev_kernel and mlp_adam_planes_kernel so both round identically
+// one element of the device-step Adam; shared by adam_dev_kernel and mlp_adam_planes_kernel so both round identically.
+// torch.optim.Adam, single-tensor form (amsgrad off): exp_avg.lerp_(g, 1 - b1); exp_avg_sq = b2 v + (1 - b2) g g;
+// denom = sqrt(v) / sqrt(1 - b2^t) + eps; theta -= lr / (1 - b1^t) * m / denom
 __device__ __forceinline__ float adam_dev_element(float* __restrict__ theta, const float* __restrict__ grad, float* __restrict__ m,
                                                   float* __restrict__ v, size_t i, float b1, float b2, float eps, float wd,
                                                   float step_size, float bc2_sqrt)
@@ -587,17 +547,6 @@ B2_EXPORT int b200pose_colsum(const float* x, int32_t rows, int32_t cols, int32_
     return B200POSE_OK;
 }
 
-B2_EXPORT int b200pose_fold_attention(const float* w2, int32_t ld_w2, const float* b2, const float* attn_l, const float* attn_r,
-                                      int32_t heads, int32_t dim, int32_t din, float* w2e, int32_t ld_w2e, float* b2e, void* stream)
-{
-    B2_CHECK_ARG(w2 && b2 && attn_l && attn_r && w2e && b2e, "fold_attention: null argument");
-    B2_CHECK_ARG(heads >= 1 && dim >= 1 && din >= 1 && ld_w2 >= din && ld_w2e >= din, "fold_attention: bad shape");
-    const long long total = (long long)(heads * dim + 2 * heads) * (din + 1);
-    fold_attention_kernel<<<(int)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(w2, ld_w2, b2, attn_l, attn_r, heads, dim, din, w2e, ld_w2e, b2e);
-    B2_CHECK_LAUNCH();
-    return B200POSE_OK;
-}
-
 B2_EXPORT int b200pose_mse_sigmoid(const float* scores, int32_t n_nodes, const int32_t* idx, const float* labels, int32_t m,
                                    float* loss, float* dlogit, void* stream)
 {
@@ -614,18 +563,6 @@ B2_EXPORT int b200pose_sigmoid_bwd(const float* scores, const float* dscores, in
     B2_CHECK_ARG(scores && dscores && dlogit && n >= 0, "sigmoid_bwd: bad argument");
     if (n == 0) return B200POSE_OK;
     sigmoid_bwd_kernel<<<ceil_div(n, 256), 256, 0, (cudaStream_t)stream>>>(scores, dscores, n, dlogit);
-    B2_CHECK_LAUNCH();
-    return B200POSE_OK;
-}
-
-B2_EXPORT int b200pose_adam_step(float* theta, const float* grad, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
-                                 float eps, float weight_decay, int32_t step, void* stream)
-{
-    B2_CHECK_ARG(theta && grad && m && v && n >= 0 && step >= 1, "adam_step: bad argument");
-    if (n == 0) return B200POSE_OK;
-    const double bc1 = 1.0 - pow((double)beta1, (double)step), bc2 = 1.0 - pow((double)beta2, (double)step);
-    adam_kernel<<<(int)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(theta, grad, m, v, (long long)n, beta1, beta2, eps, weight_decay,
-                                                                          (float)((double)lr / bc1), (float)sqrt(bc2));
     B2_CHECK_LAUNCH();
     return B200POSE_OK;
 }

@@ -127,10 +127,8 @@ int b200pose_node_features(int32_t n_frames, int32_t n_heads_total, int32_t n_no
  * 256-row tiles above 512 rows, single CTAs below); m <= 8 rows (the pose MLP of a live frame) go to a weight-streaming
  * kernel that keeps A in registers and splits k over the lanes of a CTA, 9..16 rows to one that stages A in shared memory
  * and gives every warp an output column - either way every hi/lo weight is read once;
- * 4 / 5 / 6 / 7 force single CTAs / CTA pairs / full-width single-tile CTA pairs (256 < n <= 512; measured slower, kept
- * for A/B runs) / the few-row kernels;
- * 1 = fp32 SIMT kernel, 2 = tcgen05 kernel with tiles filled by ordinary stores, 3 = first one-tile-per-CTA
- * kernel - these three exist only for the kernel self-test.
+ * 4 / 5 / 7 force single CTAs / CTA pairs / the few-row kernels (m <= 16; more rows go to the dispatch's persistent kernel).
+ * Any other value is refused with B200POSE_E_INVALID.
  * ------------------------------------------------------------------------------------------- */
 int b200pose_linear(const uint16_t* a_hi, const uint16_t* a_lo, int32_t lda,
                     const uint16_t* w_hi, const uint16_t* w_lo, int32_t ldw,
@@ -306,13 +304,12 @@ int b200pose_transpose_planes(const uint16_t* hi, const uint16_t* lo, int32_t ro
 /* out[j] = sum_r x[r, j] * (w ? w[r, j / group] : 1): bias gradients; d attn[h, d] = sum_u d a[u, h] ft2[u, h, d] */
 int b200pose_colsum(const float* x, int32_t rows, int32_t cols, int32_t ld, const float* w, int32_t ld_w, int32_t group,
                     float* out, void* stream);
-/* w2e [heads*dim + 2*heads, ld_w2e] = [W2 ; sum_d attn_l[h,d] W2[h*dim+d, :] ; same with attn_r], b2e likewise (gat2.py:55-58
- * as one projection; the inference path does this fold once on the host, a training step after every parameter update) */
-int b200pose_fold_attention(const float* w2, int32_t ld_w2, const float* b2, const float* attn_l, const float* attn_r,
-                            int32_t heads, int32_t dim, int32_t din, float* w2e, int32_t ld_w2e, float* b2e, void* stream);
-/* The two calls above for a whole layer in one launch each: every operand plane of a layer from its fp32 parameters (W1 and
- * W1^T planes, [W2 ; folds] planes + folded bias, W2^T planes; ld_w1 = ld_w2 = round_up(din, 64)), and the three column sums
- * behind b200pose_gat_aggregate_bwd (d attn_l, d attn_r, d fc2.bias) in one pass over z and dz. */
+/* A whole layer in one launch each. b200pose_gat_prepare_layer: every operand plane of a layer from its fp32 parameters (W1 and
+ * W1^T planes, [W2 ; folds] planes + folded bias b2e, W2^T planes; ld_w1 = ld_w2 = round_up(din, 64)), where
+ * [W2 ; folds] = [W2 ; sum_d attn_l[h,d] W2[h*dim+d, :] ; same with attn_r] and b2e likewise (gat2.py:55-58 as one projection;
+ * the inference path does this fold once on the host, a training step after every parameter update).
+ * b200pose_gat_attn_bias_grad: the three column sums behind b200pose_gat_aggregate_bwd (d attn_l, d attn_r, d fc2.bias) in one
+ * pass over z and dz. */
 int b200pose_gat_prepare_layer(const float* w1, const float* w2, int32_t ld_w, const float* b2, const float* attn_l,
                                const float* attn_r, int32_t heads, int32_t dim, int32_t din,
                                uint16_t* w1_hi, uint16_t* w1_lo, int32_t ld_w1, uint16_t* w1t_hi, uint16_t* w1t_lo, int32_t ld_w1t,
@@ -331,10 +328,8 @@ int b200pose_mse_sigmoid(const float* scores, int32_t n_nodes, const int32_t* id
                          float* loss, float* dlogit, void* stream);
 /* dlogit = dscores * s * (1 - s): the final sigmoid when the loss is computed by the caller (autograd drop-in) */
 int b200pose_sigmoid_bwd(const float* scores, const float* dscores, int32_t n, float* dlogit, void* stream);
-/* torch.optim.Adam (train_skeleton_matching.py:150), single-tensor form, over one flat parameter buffer; step counts from 1 */
-int b200pose_adam_step(float* theta, const float* grad, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
-                       float eps, float weight_decay, int32_t step, void* stream);
-/* The same with the step count kept on the device: *step_dev is advanced by one and the bias corrections are computed there
+/* torch.optim.Adam (train_skeleton_matching.py:150), single-tensor form, over one flat parameter buffer, with the step count
+ * kept on the device: *step_dev is advanced by one and the bias corrections are computed there
  * (scalars_dev: 2 floats of scratch), so a whole optimisation step - forward, loss, backward, this - is replayable as a CUDA graph */
 int b200pose_adam_step_dev(float* theta, const float* grad, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
                            float eps, float weight_decay, int32_t* step_dev, float* scalars_dev, void* stream);

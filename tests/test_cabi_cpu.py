@@ -40,6 +40,17 @@ def test_argument_errors_are_reported_not_fatal():
         libmod.check(rc, 'linear')
 
 
+@pytest.mark.parametrize('impl', [1, 2, 3, 6, 9])
+def test_linear_refuses_unknown_impl(impl):
+    """b200pose_linear takes impl 0 (dispatch), 4, 5 or 7 only. Anything else is refused before any launch, so the dummy
+    pointers below are never dereferenced, with or without a GPU."""
+    L = libmod.lib()
+    p = ctypes.c_void_p(0x1000)                  # non-null, 16-byte aligned
+    rc = L.b200pose_linear(p, p, 64, p, p, 64, p, 4, 64, 64, 1.0, 1.0, p, 64, p, p, 64, impl, None)
+    assert rc == -1
+    assert re.search(rb'impl must be 0 .*4 .*5 .*or 7 ', L.b200pose_last_error())
+
+
 def test_pipeline_refuses_to_run_without_cuda():
     import torch
     if torch.cuda.is_available():
