@@ -23,9 +23,8 @@ from typing import Optional
 import numpy as np
 import torch
 
-from .pipeline import DeviceBatch, GraphArrays, HostBatch, PosePipeline, person_capacity, check, ptr
-
-_NAMES = ('sk_xy', 'sk_vp', 'sk_mask', 'sk_cam', 'head_off', 'node_off')
+from .pipeline import (INPUT_NAMES, GraphArrays, HostBatch, PosePipeline, capture_capacity, copy_inputs, person_capacity,
+                       pinned_results)
 
 
 class _Entry:
@@ -162,39 +161,29 @@ class LiveFrames:
         cfg = pipe.cfg
         ent = _Entry()
         ent.key, ent.gen, ent.has_mlp = key, 0, pipe.mlp is not None
-        pin = lambda t: torch.empty_like(t).pin_memory()
-        ent.h_in = {n: pin(getattr(hb, n)) for n in _NAMES}
-        d_in = {n: torch.empty_like(getattr(hb, n), device=dev) for n in _NAMES}
-        for n in _NAMES:
-            ent.h_in[n].copy_(getattr(hb, n))
-        ent.h_in_np = {n: ent.h_in[n].numpy() for n in _NAMES}
+        h_in, db = hb.static_copy(dev)
+        ent.h_in, ent.db = h_in, db
+        ent.h_in_np = {n: h_in[n].numpy() for n in INPUT_NAMES}
         ent.h_in_np['sk_mask'] = ent.h_in_np['sk_mask'].view(np.uint32)
-        db = DeviceBatch(1, pb.n_heads, pb.n_nodes, pb.max_heads, pb.max_enodes, d_in['sk_xy'], d_in['sk_vp'], d_in['sk_mask'],
-                         d_in['sk_cam'], d_in['head_off'], d_in['node_off'])
-        ent.db, ent.d_in = db, d_in
         p_bound = person_capacity(pb.n_heads, cfg.min_number_of_views)
-        seen = self.person_hint.get(key, 0)
-        ent.p_max = p_max = min(p_bound, max(8, (int(max(seen, p_bound // 2) * 1.25) + 7) // 8 * 8))
+        ent.p_max = p_max = capture_capacity(max(self.person_hint.get(key, 0), p_bound // 2), p_bound)
         mk = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory()
         n_out = pipe.mlp[-1]['n'] if ent.has_mlp else 0
-        ent.h_out = dict(n_persons=mk((1,), torch.int32), person_heads=mk((pb.n_heads, cfg.V_sm), torch.int32),
-                         person_sk=mk((p_max, cfg.n_cameras), torch.int32), valid=mk((p_max,), torch.uint8),
-                         enc=mk((p_max, cfg.mlp_in), torch.float32), joints=mk((p_max, max(n_out, 1)), torch.float32))
+        ent.h_out = dict(pinned_results(1, p_max, cfg.n_cameras, n_out), person_heads=mk((pb.n_heads, cfg.V_sm), torch.int32),
+                         enc=mk((p_max, cfg.mlp_in), torch.float32))
         self.sync()
         cur = torch.cuda.current_stream(dev)
         self.stream.wait_stream(cur)
         with torch.cuda.stream(self.stream):
             # eager warm-up of this shape on the side stream: workspaces, function attributes, allocator
-            for n in _NAMES:
-                d_in[n].copy_(ent.h_in[n], non_blocking=True)
+            copy_inputs(db, h_in)
             res = pipe.stage_a(db, with_coo=True)
             if ent.has_mlp:
                 pipe._stage_b_static(db, res, p_bound, p_max)
             self.stream.synchronize()
             ent.g1, ent.g2, ent.g3 = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
             with torch.cuda.graph(ent.g1, stream=self.stream):
-                for n in _NAMES:
-                    d_in[n].copy_(ent.h_in[n], non_blocking=True)
+                copy_inputs(db, h_in)
                 res = pipe.stage_a(db, with_coo=True)
                 # the dense N x F feature matrix the reference hands around as `ndata['h']`: nothing on this path reads it
                 # (layer 0 runs on the compact rows), but the driver passes it back to the model, so it is kept materialised -
@@ -204,13 +193,8 @@ class LiveFrames:
                 ent.h_out['person_heads'].copy_(res['person_heads'][: pb.n_heads], non_blocking=True)
             ent.arrays, ent.scores, ent.res = res['graph'], res['scores'], res
             if ent.has_mlp:
-                Cn = cfg.n_cameras
                 with torch.cuda.graph(ent.g2, stream=self.stream):
-                    person_sk = torch.full((p_bound, Cn), -1, dtype=torch.int32, device=dev)
-                    person_frame = torch.zeros(p_bound, dtype=torch.int32, device=dev)
-                    check(pipe.L.b200pose_gather_persons(1, ptr(db.head_off), ptr(res['person_heads']), ptr(res['n_persons']),
-                                                         ptr(res['person_off']), 0, ptr(db.sk_cam), cfg.V_sm, pipe.cams.ref,
-                                                         ptr(person_sk), ptr(person_frame), pipe._stream()), 'gather_persons')
+                    person_sk, person_frame = pipe.person_list(db, res, p_bound, fill=True)
                     x, valid, xf = pipe.encode_persons(db, p_max, person_sk, want_f32=True)
                     ent.h_out['person_sk'].copy_(person_sk[:p_max], non_blocking=True)
                     ent.h_out['valid'].copy_(valid, non_blocking=True)
@@ -220,5 +204,5 @@ class LiveFrames:
                     ent.h_out['joints'][:, :n_out].copy_(joints, non_blocking=True)
                 ent.xf, ent.joints, ent.keep3 = xf, joints, (person_sk, person_frame, x, valid)
             ent.ev_a, ent.ev_b, ent.ev_c = torch.cuda.Event(), torch.cuda.Event(), torch.cuda.Event()
-            ent.keep = list(pipe._ws.values())     # the graphs bake in workspace addresses: keep them alive
+            ent.keep = list(pipe._own.ws.values())     # the graphs bake in workspace addresses: keep them alive
         return ent

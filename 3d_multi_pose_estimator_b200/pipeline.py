@@ -31,6 +31,43 @@ def person_capacity(n_heads: int, min_views: int) -> int:
     return max(n_heads // max(int(min_views), 1), 1)
 
 
+def capture_capacity(seen: int, p_bound: int) -> int:
+    """Rows the encoder and the MLP of a captured step are sized for: the persons a shape showed, with head-room, in
+    multiples of 8 rows (the weight-stream kernel's step), at most p_bound (person_capacity of the shape). A replay that
+    finds more persons than that is redone eagerly and re-captured."""
+    return min(p_bound, max(8, (int(seen * 1.25) + 7) // 8 * 8))
+
+
+# the arrays of a packed batch that go to the device, in upload order (the tensor fields of HostBatch and DeviceBatch)
+INPUT_NAMES = ('sk_xy', 'sk_vp', 'sk_mask', 'sk_cam', 'head_off', 'node_off')
+
+
+def pinned_results(n_frames: int, rows: int, n_cameras: int, n_out: int) -> dict:
+    """Pinned host buffers for the results of a batch: per-frame person counts and offsets, and `rows` person rows."""
+    mk = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory()
+    return dict(n_persons=mk((n_frames,), torch.int32), person_off=mk((n_frames + 1,), torch.int32),
+                person_sk=mk((rows, n_cameras), torch.int32), joints=mk((rows, max(n_out, 1)), torch.float32),
+                valid=mk((rows,), torch.uint8))
+
+
+def copy_person_rows(out: dict, res: dict, P: int, p0: int = 0):
+    """Enqueues the device->host copies of the first P person rows of a result (person list, and joints and valid when
+    the result has them) into rows p0.. of a pinned_results() set, on the current stream."""
+    out['person_sk'][p0:p0 + P].copy_(res['person_sk'][:P], non_blocking=True)
+    if 'joints' in res:
+        out['joints'][p0:p0 + P].copy_(res['joints'][:P], non_blocking=True)
+        out['valid'][p0:p0 + P].copy_(res['valid'][:P], non_blocking=True)
+
+
+def host_results(bufs: dict, P: int, with_mlp: bool) -> dict:
+    """The host result of a batch with P persons, as views of a pinned_results() set."""
+    out = dict(n_persons=bufs['n_persons'], person_off=bufs['person_off'], person_sk=bufs['person_sk'][:P], n_persons_total=P)
+    if with_mlp:
+        out['joints'] = bufs['joints'][:P]
+        out['valid'] = bufs['valid'][:P]
+    return out
+
+
 class Planes:
     """An fp32 matrix stored as hi/lo bf16 planes [rows, ld] (ld multiple of 64), zero padded."""
 
@@ -168,11 +205,7 @@ class HostBatch:
         key = (n_cameras, n_out, min_views)
         cache = self.__dict__.setdefault('_results', {})
         if key not in cache:
-            B, Pmax = self.pb.n_frames, person_capacity(self.pb.n_heads, min_views)
-            mk = lambda shape, dt: (torch.empty(shape, dtype=dt).pin_memory() if torch.cuda.is_available() else torch.empty(shape, dtype=dt))
-            cache[key] = dict(n_persons=mk((B,), torch.int32), person_off=mk((B + 1,), torch.int32),
-                              person_sk=mk((Pmax, n_cameras), torch.int32), joints=mk((Pmax, max(n_out, 1)), torch.float32),
-                              valid=mk((Pmax,), torch.uint8))
+            cache[key] = pinned_results(self.pb.n_frames, person_capacity(self.pb.n_heads, min_views), n_cameras, n_out)
         return cache[key]
 
     def to_device(self, device) -> DeviceBatch:
@@ -181,6 +214,34 @@ class HostBatch:
         return DeviceBatch(pb.n_frames, pb.n_heads, pb.n_nodes, pb.max_heads, pb.max_enodes,
                            cp(self.sk_xy), cp(self.sk_vp), cp(self.sk_mask), cp(self.sk_cam), cp(self.head_off), cp(self.node_off),
                            host_offsets=(np.asarray(pb.head_off, dtype=np.int64), np.asarray(pb.node_off, dtype=np.int64)))
+
+    def upload(self, device, copy_stream, consumer):
+        """to_device() enqueued on `copy_stream` for compute on `consumer`: returns the DeviceBatch and an event recorded
+        after its copies, which the consumer waits for."""
+        with torch.cuda.stream(copy_stream):
+            db = self.to_device(device)
+            for n in INPUT_NAMES:
+                getattr(db, n).record_stream(consumer)
+            ev = torch.cuda.Event()
+            ev.record(copy_stream)
+        return db, ev
+
+    def static_copy(self, device):
+        """(h_in, db) for a captured step that uploads its own inputs (copy_inputs): pinned staging buffers holding this
+        batch's arrays, and a DeviceBatch of device buffers of the same shapes. The graph bakes in the addresses of both, so
+        a replay takes new frames of the shape through h_in."""
+        h_in = {n: torch.empty_like(getattr(self, n)).pin_memory() for n in INPUT_NAMES}
+        d_in = [torch.empty_like(getattr(self, n), device=device) for n in INPUT_NAMES]
+        for n in INPUT_NAMES:
+            h_in[n].copy_(getattr(self, n))
+        pb = self.pb
+        return h_in, DeviceBatch(pb.n_frames, pb.n_heads, pb.n_nodes, pb.max_heads, pb.max_enodes, *d_in)
+
+
+def copy_inputs(db: DeviceBatch, h_in: dict):
+    """Enqueues the host->device copies of a batch's inputs from the staging buffers of HostBatch.static_copy()."""
+    for n in INPUT_NAMES:
+        getattr(db, n).copy_(h_in[n], non_blocking=True)
 
 
 class GraphArrays:
@@ -210,11 +271,25 @@ def _on_own_device(fn):
 
     @functools.wraps(fn)
     def wrapper(self, *a, **k):
-        if torch.cuda.current_device() == self._dev_index_checked():
+        if torch.cuda.current_device() == self._device_index():
             return fn(self, *a, **k)
         with torch.cuda.device(self.device):
             return fn(self, *a, **k)
     return wrapper
+
+
+class _Owned:
+    """The streams and caches of one pipeline. A twin() gets a fresh set, so two lanes share nothing but the read-only
+    camera tables and weight planes."""
+
+    def __init__(self):
+        self.ws = {}                                 # activation workspaces (planes_ws, f32_ws)
+        self.streams = {}                            # auxiliary streams by role, created on first use (_aux_stream)
+        self.lanes = None                            # lanes(): (weights generation, pipelines, streams)
+        self.graphs = collections.OrderedDict()      # infer_host_graph: captured step per batch shape
+        self.graph_person_hint = {}                  # infer_host_graph: the largest person count a shape has shown
+        self.stream_results = {}                     # infer_host_stream: rotating pinned result sets per batch size
+        self.person_stage = {}                       # encode_person_dicts: pinned + device staging buffers per size
 
 
 class PosePipeline:
@@ -238,7 +313,7 @@ class PosePipeline:
         self.fuse_small_fc2 = True  # last GAT layer: fc2 (3 columns) inside fc1's epilogue (False: two launches, for A/B runs)
         self.threshold = float(threshold)
         self.launches = 0
-        self._ws = {}
+        self._own = _Owned()
         with torch.cuda.device(self.device):
             self.cams = DeviceCameras(cfg, self.device)
             self.gat = self.prepare_gat(gat_state) if gat_state is not None else None
@@ -264,34 +339,40 @@ class PosePipeline:
         self._mlp = layers
         self._weights_gen = getattr(self, '_weights_gen', 0) + 1
 
-    def _dev_index_checked(self):
+    def _device_index(self) -> int:
         if self._dev_index is None:
             self._dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
         return self._dev_index
 
+    def _aux_stream(self, role: str):
+        """This pipeline's stream for `role` ('side', 'copy', 'd2h', 'counts'), created on first use. Streams map
+        round-robin onto the hardware queues, so one created before it is needed can alias a stream that is in use."""
+        s = self._own.streams.get(role)
+        if s is None:
+            s = self._own.streams[role] = torch.cuda.Stream(self.device)
+        return s
+
     # ------------------------------------------------------------------ compute lanes
     def twin(self) -> "PosePipeline":
         """A second pipeline on the same device that SHARES this one's camera tables and weight planes (read-only) and has its
-        own workspaces, side stream and caches: two independent batches can then be in flight on two CUDA streams. A step
+        own workspaces, streams and caches: two independent batches can then be in flight on two CUDA streams. A step
         has ~0.26 ms of latency-bound phases (graph build + features, clustering, person list, encoder: 8-26 % warps
         active) that fit beside another batch's tensor-core GEMMs on the same SMs."""
         t = PosePipeline.__new__(PosePipeline)
         t.__dict__.update(self.__dict__)
-        t._ws = {}
+        t._own = _Owned()
         t.launches = 0
-        for k in ('_side_stream', '_copy_stream', '_d2h_stream', '_stream_results', '_graphs', '_graph_person_hint', '_person_stage', '_lanes'):
-            t.__dict__.pop(k, None)
         return t
 
     def lanes(self, n: int):
         """[self, twin, ...] and one compute stream per extra lane (lane 0 runs on the caller's current stream); cached.
         A lane whose weights were replaced on `self` since it was made is rebuilt."""
-        have = self.__dict__.get('_lanes')
+        have = self._own.lanes
         gen = getattr(self, '_weights_gen', 0)
         if have is None or have[0] != gen or len(have[1]) < n:
             pipes = [self] + [self.twin() for _ in range(n - 1)]
             streams = [None] + [torch.cuda.Stream(self.device) for _ in range(n - 1)]
-            have = self.__dict__['_lanes'] = (gen, pipes, streams)
+            have = self._own.lanes = (gen, pipes, streams)
         return have[1][:n], have[2][:n]
 
     # ------------------------------------------------------------------ workspace
@@ -299,30 +380,28 @@ class PosePipeline:
         """Activation planes from a per-pipeline workspace. They are zero-initialised once; kernels write
         every valid column and only ever write zeros into the K padding, so reuse needs no memset."""
         key = (tag, round_up(max(cols, 1), 64))
-        ws = self._ws.get(key)
+        ws = self._own.ws.get(key)
         if ws is None or ws.hi.shape[0] < rows:
             cap = max(rows, int(ws.hi.shape[0] * 1.25) if ws is not None else rows)
             ws = Planes(cap, cols, self.device)
-            self._ws[key] = ws
+            self._own.ws[key] = ws
         view = Planes.__new__(Planes)
         view.rows, view.cols, view.ld, view.hi, view.lo = rows, cols, ws.ld, ws.hi, ws.lo
         return view
 
     def f32_ws(self, tag: str, rows: int, cols: int) -> torch.Tensor:
         key = (tag, cols)
-        t = self._ws.get(key)
+        t = self._own.ws.get(key)
         if t is None or t.shape[0] < rows:
             t = torch.empty((max(rows, 1), cols), dtype=torch.float32, device=self.device)
-            self._ws[key] = t
+            self._own.ws[key] = t
         return t
 
     # ------------------------------------------------------------------ weights
     def _stream(self):
         # the raw cudaStream_t of torch's current stream on this device; the public torch.cuda.current_stream() costs
         # ~17 us per call (device-index resolution), which at 30 launches is most of a live frame's host time
-        if self._dev_index is None:
-            self._dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
-        return C.c_void_p(torch._C._cuda_getCurrentRawStream(self._dev_index))
+        return C.c_void_p(torch._C._cuda_getCurrentRawStream(self._device_index()))
 
     def prepare_gat(self, st, residual: bool = False):
         """Split every projection into planes; fold the attention vectors into fc2 as 2*heads extra output
@@ -403,9 +482,7 @@ class PosePipeline:
         self.launches += 1
         if overlap:
             cur = torch.cuda.current_stream(self.device)
-            side = self.__dict__.get('_side_stream')
-            if side is None:
-                side = self.__dict__['_side_stream'] = torch.cuda.Stream(self.device)
+            side = self._aux_stream('side')
             side.wait_stream(cur)                               # the packed batch (and, in a capture, the fork point)
             with torch.cuda.stream(side):
                 check(self.L.b200pose_build_graph(db.n_frames, ptr(db.head_off), ptr(db.node_off), ptr(db.sk_cam), self.cams.ref,
@@ -535,21 +612,20 @@ class PosePipeline:
                  ptr(person_heads), ptr(n_persons), self._stream()), 'cluster')
         return person_heads, n_persons[: db.n_frames]
 
-    def gather_persons(self, db: DeviceBatch, person_heads, n_persons):
-        """Dense person list. One 4-byte device->host read (the person count sizes the MLP launch)."""
-        person_off = torch.empty(db.n_frames + 1, dtype=torch.int32, device=self.device)
-        self.launches += 1
-        check(self.L.b200pose_gather_persons(db.n_frames, ptr(db.head_off), ptr(person_heads), ptr(n_persons), ptr(person_off), 1,
-                                             ptr(db.sk_cam), self.cfg.V_sm, self.cams.ref, None, None, self._stream()), 'scan')
-        P = int(person_off[db.n_frames].item())
-        Cn = self.cfg.n_cameras
-        person_sk = torch.empty((max(P, 1), Cn), dtype=torch.int32, device=self.device)
-        person_frame = torch.empty(max(P, 1), dtype=torch.int32, device=self.device)
-        self.launches += 1
-        check(self.L.b200pose_gather_persons(db.n_frames, ptr(db.head_off), ptr(person_heads), ptr(n_persons), ptr(person_off), 0,
-                                             ptr(db.sk_cam), self.cfg.V_sm, self.cams.ref, ptr(person_sk), ptr(person_frame),
-                                             self._stream()), 'gather_persons')
-        return P, person_off, person_sk[:P], person_frame[:P]
+    def person_list(self, db: DeviceBatch, res: dict, rows: int, fill: bool = False):
+        """The persons stage_a found as person_sk [rows, C] (skeleton id per camera, -1 = none) and person_frame [rows];
+        `rows` must cover the person count. With fill=True the rows past the count are person_sk = -1, person_frame = 0."""
+        n, i32 = max(rows, 1), dict(dtype=torch.int32, device=self.device)
+        if fill:
+            person_sk, person_frame = torch.full((n, self.cfg.n_cameras), -1, **i32), torch.zeros(n, **i32)
+        else:
+            person_sk, person_frame = torch.empty((n, self.cfg.n_cameras), **i32), torch.empty(n, **i32)
+        if rows > 0:
+            self.launches += 1
+            check(self.L.b200pose_gather_persons(db.n_frames, ptr(db.head_off), ptr(res['person_heads']), ptr(res['n_persons']),
+                                                 ptr(res['person_off']), 0, ptr(db.sk_cam), self.cfg.V_sm, self.cams.ref,
+                                                 ptr(person_sk), ptr(person_frame), self._stream()), 'gather_persons')
+        return person_sk, person_frame
 
     def encode_persons(self, db: DeviceBatch, P: int, person_sk, want_f32=False, n_dev: Optional[torch.Tensor] = None):
         """MLP input rows of P persons. With `n_dev` (int32 device scalar) P is a capacity and the kernel handles the
@@ -597,7 +673,7 @@ class PosePipeline:
         for nb in (n_xy, n_vp, n_mask, n_psk):                  # every region starts 8-byte aligned
             offs.append((offs[-1] + nb + 7) // 8 * 8)
         total = offs[-1]
-        stage = self.__dict__.setdefault('_person_stage', {})
+        stage = self._own.person_stage
         if total not in stage:
             stage[total] = (torch.empty(total, dtype=torch.uint8).pin_memory(), torch.empty(total, dtype=torch.uint8, device=self.device))
         h_buf, d_buf = stage[total]
@@ -688,14 +764,7 @@ class PosePipeline:
         """Stage 3 of a batch. Reads the person count back (one 4-byte device->host copy: it sizes the launches),
         then person list, MLP-input encoder and MLP."""
         P = int(res['person_off'][db.n_frames].item()) if db.n_heads > 0 else 0
-        Cn = self.cfg.n_cameras
-        person_sk = torch.empty((max(P, 1), Cn), dtype=torch.int32, device=self.device)
-        person_frame = torch.empty(max(P, 1), dtype=torch.int32, device=self.device)
-        if P > 0:
-            self.launches += 1
-            check(self.L.b200pose_gather_persons(db.n_frames, ptr(db.head_off), ptr(res['person_heads']), ptr(res['n_persons']),
-                                                 ptr(res['person_off']), 0, ptr(db.sk_cam), self.cfg.V_sm, self.cams.ref,
-                                                 ptr(person_sk), ptr(person_frame), self._stream()), 'gather_persons')
+        person_sk, person_frame = self.person_list(db, res, P)
         res.update(person_sk=person_sk[:P], person_frame=person_frame[:P], n_persons_total=P)
         if self.mlp is not None:
             if P > 0:
@@ -717,13 +786,7 @@ class PosePipeline:
         if db.n_heads == 0 or self.mlp is None:
             return self.stage_b(db, res)
         cap = person_capacity(db.n_heads, self.cfg.min_number_of_views)
-        Cn = self.cfg.n_cameras
-        person_sk = torch.empty((cap, Cn), dtype=torch.int32, device=self.device)
-        person_frame = torch.empty(cap, dtype=torch.int32, device=self.device)
-        self.launches += 1
-        check(self.L.b200pose_gather_persons(db.n_frames, ptr(db.head_off), ptr(res['person_heads']), ptr(res['n_persons']),
-                                             ptr(res['person_off']), 0, ptr(db.sk_cam), self.cfg.V_sm, self.cams.ref,
-                                             ptr(person_sk), ptr(person_frame), self._stream()), 'gather_persons')
+        person_sk, person_frame = self.person_list(db, res, cap)
         n_dev = res['person_off'][db.n_frames:db.n_frames + 1]
         x, valid, _ = self.encode_persons(db, cap, person_sk, n_dev=n_dev)
         joints = self.mlp_forward(x, cap, m_dev=n_dev)
@@ -759,46 +822,33 @@ class PosePipeline:
         compute use infer_host_stream(), which prefetches the NEXT batch instead. Results are in frame order."""
         chunks = hb.split(n_chunks)
         cur = torch.cuda.current_stream(self.device)
-        if getattr(self, '_copy_stream', None) is None:
-            self._copy_stream = torch.cuda.Stream(self.device)
-        cs = self._copy_stream
+        cs = self._aux_stream('copy')
         cs.wait_stream(cur)
-        dbs, evs = [], []
-        with torch.cuda.stream(cs):
-            for ch in chunks:
-                db = ch.to_device(self.device)
-                for t in (db.sk_xy, db.sk_vp, db.sk_mask, db.sk_cam, db.head_off, db.node_off):
-                    t.record_stream(cur)
-                ev = torch.cuda.Event()
-                ev.record(cs)
-                dbs.append(db); evs.append(ev)
+        uploads = [ch.upload(self.device, cs, cur) for ch in chunks]
         out_bufs = hb.result_buffers(self.cfg.n_cameras, self.mlp[-1]['n'] if self.mlp is not None else 0, self.cfg.min_number_of_views)
         parts = []
         p_base = 0
 
         def finish(i):
             nonlocal p_base
-            db, ch = dbs[i], chunks[i]
+            db, ch = uploads[i][0], chunks[i]
             res = self.stage_b(db, staged[i])
             P = res['n_persons_total']
             f0, f1 = ch.frame_range
             out_bufs['n_persons'][f0:f1].copy_(res['n_persons'], non_blocking=True)
             out_bufs['person_off'][f0:f1 + 1].copy_(res['person_off'], non_blocking=True)
             if P > 0:
-                out_bufs['person_sk'][p_base:p_base + P].copy_(res['person_sk'], non_blocking=True)
-                if 'joints' in res:
-                    out_bufs['joints'][p_base:p_base + P].copy_(res['joints'], non_blocking=True)
-                    out_bufs['valid'][p_base:p_base + P].copy_(res['valid'], non_blocking=True)
+                copy_person_rows(out_bufs, res, P, p_base)
             parts.append((f0, f1, p_base, P, ch.head_range[0]))
             p_base += P
 
         staged = []
-        for i, db in enumerate(dbs):
-            cur.wait_event(evs[i])
+        for i, (db, ev) in enumerate(uploads):
+            cur.wait_event(ev)
             staged.append(self.stage_a(db))
             if i >= 1:
                 finish(i - 1)
-        finish(len(dbs) - 1)
+        finish(len(uploads) - 1)
         cur.synchronize()
         # chunk-local -> batch-global indices (host side, a few KB)
         P_tot = p_base
@@ -812,12 +862,7 @@ class PosePipeline:
             if h0:
                 blk = person_sk[pb0:pb0 + P]
                 blk[blk >= 0] += h0
-        out = dict(n_persons=out_bufs['n_persons'], person_off=out_bufs['person_off'], person_sk=out_bufs['person_sk'][:P_tot],
-                   n_persons_total=P_tot)
-        if self.mlp is not None:
-            out['joints'] = out_bufs['joints'][:P_tot]
-            out['valid'] = out_bufs['valid'][:P_tot]
-        return out
+        return host_results(out_bufs, P_tot, self.mlp is not None)
 
     # ------------------------------------------------------------------ low-latency path: one CUDA graph per batch shape
     def _stage_b_static(self, db: DeviceBatch, res: dict, p_bound: int, p_max: int):
@@ -825,16 +870,11 @@ class PosePipeline:
         persons (disjoint components of at least that many heads), the encoder and the MLP for p_max <= p_bound rows; rows past the real count keep person_sk = -1,
         encode to zero rows with valid = 0 and are dropped on the host. This is what lets the whole step live in one CUDA
         graph."""
-        Cn = self.cfg.n_cameras
-        person_sk = torch.full((p_bound, Cn), -1, dtype=torch.int32, device=self.device)
-        person_frame = torch.zeros(p_bound, dtype=torch.int32, device=self.device)
-        self.launches += 1
-        check(self.L.b200pose_gather_persons(db.n_frames, ptr(db.head_off), ptr(res['person_heads']), ptr(res['n_persons']),
-                                             ptr(res['person_off']), 0, ptr(db.sk_cam), self.cfg.V_sm, self.cams.ref,
-                                             ptr(person_sk), ptr(person_frame), self._stream()), 'gather_persons')
+        person_sk, person_frame = self.person_list(db, res, p_bound, fill=True)
         x, valid, _ = self.encode_persons(db, p_max, person_sk)
         joints = self.mlp_forward(x, p_max)
-        return person_sk, valid, joints
+        res.update(person_sk=person_sk, person_frame=person_frame, valid=valid, joints=joints)
+        return res
 
     @_on_own_device
     def infer_host_graph(self, hb: HostBatch, max_cached: int = 64):
@@ -852,64 +892,45 @@ class PosePipeline:
         # kernel choices and the weight planes - all part of the key, so a change re-captures instead of replaying stale values
         key = (pb.n_frames, pb.n_heads, pb.n_nodes, pb.max_heads, pb.max_enodes, self.threshold, self.cfg.min_number_of_views,
                self.agg_impl, self.gemm_impl, self._weights_gen)
-        cache = self.__dict__.setdefault('_graphs', collections.OrderedDict())
+        cache = self._own.graphs
         ent = cache.get(key)
         cur = torch.cuda.current_stream(self.device)
-        names = ('sk_xy', 'sk_vp', 'sk_mask', 'sk_cam', 'head_off', 'node_off')
         if ent is None:
             warm = self.infer_host(hb)                          # eager warm-up of this shape: workspaces, function attributes
-            hint = self.__dict__.setdefault('_graph_person_hint', {})
-            seen = max(int(warm['n_persons_total']), hint.get(key, 0))
-            pin = lambda t: torch.empty_like(t).pin_memory()
-            h_in = {n: pin(getattr(hb, n)) for n in names}
-            d_in = {n: torch.empty_like(getattr(hb, n), device=self.device) for n in names}
-            db = DeviceBatch(pb.n_frames, pb.n_heads, pb.n_nodes, pb.max_heads, pb.max_enodes, d_in['sk_xy'], d_in['sk_vp'],
-                             d_in['sk_mask'], d_in['sk_cam'], d_in['head_off'], d_in['node_off'])
+            seen = max(int(warm['n_persons_total']), self._own.graph_person_hint.get(key, 0))
+            h_in, db = hb.static_copy(self.device)
             # heads // min_number_of_views bounds the person count and sizes the person list; the encoder and the MLP
-            # are captured for a tighter capacity - the count this shape showed, with head-room, in multiples of 8 rows (the
-            # weight-stream kernel's step) - and a replay that finds more persons than that is redone eagerly and re-captured
+            # are captured for the tighter capacity this shape showed
             p_bound = person_capacity(pb.n_heads, self.cfg.min_number_of_views)
-            p_max = min(p_bound, max(8, (int(seen * 1.25) + 7) // 8 * 8))
-            n_out = self.mlp[-1]['n']
-            mk = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory()
-            h_out = dict(n_persons=mk((pb.n_frames,), torch.int32), person_off=mk((pb.n_frames + 1,), torch.int32),
-                         person_sk=mk((p_max, self.cfg.n_cameras), torch.int32), joints=mk((p_max, n_out), torch.float32),
-                         valid=mk((p_max,), torch.uint8))
-            for n in names:
-                h_in[n].copy_(getattr(hb, n))
+            p_max = capture_capacity(seen, p_bound)
+            h_out = pinned_results(pb.n_frames, p_max, self.cfg.n_cameras, self.mlp[-1]['n'])
             graph = torch.cuda.CUDAGraph()
             cur.synchronize()
             with torch.cuda.graph(graph):
-                for n in names:
-                    d_in[n].copy_(h_in[n], non_blocking=True)
-                res = self.stage_a(db)
-                person_sk, valid, joints = self._stage_b_static(db, res, p_bound, p_max)
+                copy_inputs(db, h_in)
+                res = self._stage_b_static(db, self.stage_a(db), p_bound, p_max)
                 h_out['n_persons'].copy_(res['n_persons'], non_blocking=True)
                 h_out['person_off'].copy_(res['person_off'], non_blocking=True)
-                h_out['person_sk'].copy_(person_sk[:p_max], non_blocking=True)
-                h_out['joints'].copy_(joints, non_blocking=True)
-                h_out['valid'].copy_(valid, non_blocking=True)
+                copy_person_rows(h_out, res, p_max)
             # the graph bakes in device addresses: keep everything it touches alive (workspaces are replaced when a
             # larger batch makes them grow)
-            ent = dict(graph=graph, h_in=h_in, h_out=h_out, p_cap=p_max, keep=(d_in, db, res, person_sk, valid, joints, list(self._ws.values())))
+            ent = dict(graph=graph, h_in=h_in, h_out=h_out, p_cap=p_max, keep=(db, res, list(self._own.ws.values())))
             cache[key] = ent
             while len(cache) > max_cached:
                 cache.popitem(last=False)
         else:
             cache.move_to_end(key)
-            for n in names:
+            for n in INPUT_NAMES:
                 ent['h_in'][n].copy_(getattr(hb, n))
         ent['graph'].replay()
         cur.synchronize()
-        h_out = ent['h_out']
-        P = int(h_out['person_off'][pb.n_frames])
+        P = int(ent['h_out']['person_off'][pb.n_frames])
         if P > ent['p_cap']:                                    # more persons than the captured capacity: eager, and a new capture next time
-            self.__dict__.setdefault('_graph_person_hint', {})[key] = P
+            self._own.graph_person_hint[key] = P
             del cache[key]
             return self.infer_host(hb)
         # copies: the pinned buffers belong to the cached graph and the next replay of this shape overwrites them
-        return dict(n_persons=h_out['n_persons'].clone(), person_off=h_out['person_off'].clone(), person_sk=h_out['person_sk'][:P].clone(),
-                    n_persons_total=P, joints=h_out['joints'][:P].clone(), valid=h_out['valid'][:P].clone())
+        return {k: v.clone() if torch.is_tensor(v) else v for k, v in host_results(ent['h_out'], P, True).items()}
 
     @_on_own_device
     def infer_frames(self, frames):
@@ -937,13 +958,7 @@ class PosePipeline:
             from . import DEFAULT_LANES
             lanes = DEFAULT_LANES
         cur = torch.cuda.current_stream(self.device)
-        if getattr(self, '_copy_stream', None) is None:
-            self._copy_stream = torch.cuda.Stream(self.device)
-        if getattr(self, '_d2h_stream', None) is None:
-            self._d2h_stream = torch.cuda.Stream(self.device)
-        if getattr(self, '_cnt_stream', None) is None:
-            self._cnt_stream = torch.cuda.Stream(self.device)
-        cs, ds, dc = self._copy_stream, self._d2h_stream, self._cnt_stream
+        cs, ds, dc = [self._aux_stream(role) for role in ('copy', 'd2h', 'counts')]
         pipes, lane_streams = self.lanes(max(1, int(lanes)))
         depth = len(pipes)                                     # batches enqueued ahead of the one whose results the host waits for
         lane_streams = [cur if s is None else s for s in lane_streams]
@@ -960,18 +975,12 @@ class PosePipeline:
                 return None
             lane = count[0] % len(pipes)
             count[0] += 1
-            with torch.cuda.stream(cs):
-                db = hb.to_device(self.device)
-                for t in (db.sk_xy, db.sk_vp, db.sk_mask, db.sk_cam, db.head_off, db.node_off):
-                    t.record_stream(lane_streams[lane])
-                ev = torch.cuda.Event()
-                ev.record(cs)
-            return hb, db, ev, lane
+            return (hb, *hb.upload(self.device, cs, lane_streams[lane]), lane)
 
         # pinned result buffers: depth + 3 rotating sets per batch size (depth + 1 batches are in flight, and a yielded result
         # stays valid until two more batches have been yielded), owned by the pipeline - the same HostBatch may be streamed
         # repeatedly.
-        pool = self.__dict__.setdefault('_stream_results', {})
+        pool = self._own.stream_results
         turn = [0]
 
         def result_set(hb):
@@ -979,10 +988,7 @@ class PosePipeline:
             key = (B, cap, n_out, depth + 3)
             sets = pool.get(key)
             if sets is None:
-                mk = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory()
-                sets = pool[key] = [dict(n_persons=mk((B,), torch.int32), person_off=mk((B + 1,), torch.int32),
-                                         person_sk=mk((cap, self.cfg.n_cameras), torch.int32), joints=mk((cap, max(n_out, 1)), torch.float32),
-                                         valid=mk((cap,), torch.uint8)) for _ in range(depth + 3)]
+                sets = pool[key] = [pinned_results(B, cap, self.cfg.n_cameras, n_out) for _ in range(depth + 3)]
             turn[0] += 1
             return sets[turn[0] % (depth + 3)]
 
@@ -1017,16 +1023,9 @@ class PosePipeline:
             res['n_persons_total'] = P
             if P > 0:
                 with torch.cuda.stream(ds):
-                    bufs['person_sk'][:P].copy_(res['person_sk'][:P], non_blocking=True)
-                    if 'joints' in res:
-                        bufs['joints'][:P].copy_(res['joints'][:P], non_blocking=True)
-                        bufs['valid'][:P].copy_(res['valid'][:P], non_blocking=True)
+                    copy_person_rows(bufs, res, P)
                 ds.synchronize()
-            out = dict(n_persons=bufs['n_persons'], person_off=bufs['person_off'], person_sk=bufs['person_sk'][:P], n_persons_total=P)
-            if self.mlp is not None:
-                out['joints'] = bufs['joints'][:P]
-                out['valid'] = bufs['valid'][:P]
-            return out
+            return host_results(bufs, P, self.mlp is not None)
 
         nxt = prefetch()
         pending = collections.deque()

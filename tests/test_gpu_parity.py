@@ -669,6 +669,8 @@ def test_stream_lanes_keep_order_and_results():
     held = list(pipe.infer_host_stream(hbs[:3], lanes=3))                 # three results held without copying
     for g, w in zip(held[-2:], first[1:3]):
         assert np.array_equal(np.asarray(g['joints']), w['joints'])
+    # a twin owns its streams: one made after the stream ran does not share the pipeline's counts stream
+    assert pipe.twin()._aux_stream('counts') is not pipe._aux_stream('counts')
 
 
 def test_cuda_graph_host_path_matches_eager():
@@ -695,18 +697,19 @@ def test_cuda_graph_host_path_matches_eager():
             if want['n_persons_total']:
                 assert torch.equal(got['valid'].bool(), want['valid'].bool())
                 assert (got['joints'] - want['joints']).abs().max().item() <= 1e-5
-    assert len(getattr(pipe, '_graphs')) >= 2 and len(getattr(pipe, '_graphs')) <= len(keys)
+    graphs = pipe._own.graphs
+    assert len(graphs) >= 2 and len(graphs) <= len(keys)
     # a replay that finds more persons than the captured capacity falls back to the eager path and re-captures next time
     hb = pipeline_mod.HostBatch(batches[0])
     want = {k: (v.clone() if hasattr(v, 'clone') else v) for k, v in pipe.infer_host(hb).items()}
-    key = next(k for k in pipe._graphs if k[0] == 1 and k[1] == batches[0].n_heads and k[2] == batches[0].n_nodes)
+    key = next(k for k in graphs if k[0] == 1 and k[1] == batches[0].n_heads and k[2] == batches[0].n_nodes)
     assert want['n_persons_total'] > 0
-    pipe._graphs[key]['p_cap'] = 0
+    graphs[key]['p_cap'] = 0
     got = pipe.infer_host_graph(hb)
-    assert key not in pipe._graphs and got['n_persons_total'] == want['n_persons_total']
+    assert key not in graphs and got['n_persons_total'] == want['n_persons_total']
     assert torch.equal(got['person_sk'], want['person_sk']) and torch.equal(got['joints'], want['joints'])
     got = pipe.infer_host_graph(hb)                                     # captured again, capacity from the remembered count
-    assert key in pipe._graphs and pipe._graphs[key]['p_cap'] >= want['n_persons_total']
+    assert key in graphs and graphs[key]['p_cap'] >= want['n_persons_total']
     assert torch.equal(got['person_sk'], want['person_sk']) and (got['joints'] - want['joints']).abs().max().item() <= 1e-5
 
 
