@@ -84,14 +84,15 @@ struct ClusterParams {
     int v_sm; double threshold; int min_views;
     int* person_heads; int* n_persons;
     int max_heads, max_keys, table_cap;
-    int dbg;        // b200pose_set_debug bit 128: frame 0 prints the clock of each phase
     int general;    // 1: edge-node list without closed form (b200pose_build_graph_pairs): first-seen order from the pairs
 };
 
 // blockDim = 32 (frames of a few hundred edge-nodes: everything is warp-synchronous) or 256 / 1024 (large frames: the sort
 // and the table passes use the whole CTA; the order-dependent parts still run on one lane).
+// The second launch bound sets the register budget: 64 for the 256-thread instantiation (4 CTAs), whose rank sort keeps 16
+// keys and 16 ranks per lane in registers (ptxas's own choice, 40, spills them), and 32 for the 1024-thread one (2 CTAs).
 template <int MAXT>
-__global__ void __launch_bounds__(MAXT) cluster_kernel(ClusterParams p)
+__global__ void __launch_bounds__(MAXT, MAXT == 256 ? 4 : 2) cluster_kernel(ClusterParams p)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ int n_seen_s, n_valid_s, n_links_s;
@@ -100,7 +101,6 @@ __global__ void __launch_bounds__(MAXT) cluster_kernel(ClusterParams p)
     const bool one_warp = nt == 32;
     auto bsync = [&]() { if (one_warp) __syncwarp(); else __syncthreads(); };
     const int b = blockIdx.x;
-    const long long t_start = (p.dbg & 128) ? clock64() : 0;
     const int h0 = p.head_off[b];
     const int H = p.head_off[b + 1] - h0;
     const int n0 = p.node_off[b];
@@ -280,8 +280,6 @@ __global__ void __launch_bounds__(MAXT) cluster_kernel(ClusterParams p)
     // (:90-104) forgets the absorbed group's cameras, which can revive a matching: the rest of the batch is then
     // tested again. A 10-view x 16-person frame has ~8000 matchings above the threshold and ~140 links; the walk used
     // to be one lane over all of them. ----
-    long long t_merge0 = 0;
-    if (p.dbg & 128) t_merge0 = clock64();
     int n_links = 0;
     if (tid < 32) {
         int cur = 0;
@@ -352,7 +350,6 @@ __global__ void __launch_bounds__(MAXT) cluster_kernel(ClusterParams p)
         }
     }
     bsync();
-    const long long t_merged = (p.dbg & 128) ? clock64() : 0;
 
     // ---- connected components in first-seen order, BFS by levels (:117-130) ----
     for (int h = tid; h < H; h += nt) flag[h] = 0;                               // reuse as "done"
@@ -408,9 +405,6 @@ __global__ void __launch_bounds__(MAXT) cluster_kernel(ClusterParams p)
             ++n_out;
         }
         if (lane == 0) p.n_persons[b] = n_out;
-        if ((p.dbg & 128) && b == 0 && lane == 0)
-            printf("cluster frame 0: H %d M %d matchings %d links %d | clocks: threshold+sort %lld, merge %lld, components %lld\n", H, M, n_valid,
-                   n_lk, t_merge0 - t_start, t_merged - t_merge0, clock64() - t_merged);
     }
 }
 
@@ -513,7 +507,6 @@ static int cluster_launch(int32_t n_frames, const int32_t* head_off, const int32
     ClusterParams p;
     p.head_off = head_off; p.node_off = node_off; p.pairs = pairs; p.node_cam = node_cam; p.scores = scores;
     p.v_sm = v_sm; p.threshold = threshold; p.min_views = min_views; p.person_heads = person_heads; p.n_persons = n_persons;
-    p.dbg = g_debug_flags;
     p.general = general;
     p.max_heads = max_heads_per_frame < 1 ? 1 : max_heads_per_frame;
     int keys = 1;

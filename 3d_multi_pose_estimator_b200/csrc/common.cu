@@ -3,7 +3,6 @@
 #include <string.h>
 
 namespace b200pose {
-int g_debug_flags = 0;
 static thread_local char g_err[512] = "";
 void set_error(const char* fmt, ...) {
     va_list ap;
@@ -21,9 +20,4 @@ extern "C" __attribute__((visibility("default"))) int b200pose_device_cc(void) {
     B2_CHECK_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
     B2_CHECK_CUDA(cudaDeviceGetAttribute(&minor, cudaDevAttrComputeCapabilityMinor, dev));
     return major * 10 + minor;
-}
-extern "C" __attribute__((visibility("default"))) int b200pose_set_debug(int flags) {
-    const int old = b200pose::g_debug_flags;
-    b200pose::g_debug_flags = flags;
-    return old;
 }

@@ -10,7 +10,6 @@
 namespace b200pose {
 
 void set_error(const char* fmt, ...);
-extern int g_debug_flags;          // b200pose_set_debug(): kernel bring-up switches, 0 in production
 
 #define B2_CHECK_ARG(cond, ...)                                   \
     do {                                                          \

@@ -40,7 +40,6 @@ struct AggParams {
     int stage_cap;      // large-frame kernel: z rows of shared memory per CTA
     int edge_units;     // large-frame kernel: edge-node work units per frame
     int head_units;     // large-frame kernel: head work units per frame
-    int dbg;            // b200pose_set_debug bits: 16 = no output stores, 32 = skip head contributions, 64 = skip edge-node destinations
 };
 
 template <int VEC> __device__ __forceinline__ void load_vec(const float* p, float (&v)[VEC]) {
@@ -363,7 +362,6 @@ template <> struct VecT<2> { using type = float2; };
 template <> struct VecT<1> { using type = float; };
 
 template <int VEC> __device__ __forceinline__ void store_out(const AggParams& p, bool slope_le1, int gv, int c0, const float (&v)[VEC]) {
-    if (p.dbg & 16) return;
     if (p.raw_f32) {
         float* o = p.raw_f32 + (size_t)gv * (p.heads * p.dim) + c0;
 #pragma unroll
@@ -578,7 +576,7 @@ __global__ void __launch_bounds__(kFrameThreads, 1) gat_aggregate_frame_kernel(A
         }
         // (a) the edge-node destination of this warp: in-edges (h1 -> e), (h2 -> e), (e -> e)
         const int k = k0 + wid;
-        if (k < k1 && !(p.dbg & 64)) {
+        if (k < k1) {
             const int h1 = prs[2 * k] - n0, h2 = prs[2 * k + 1] - n0;
             const float* re = rows + (size_t)(k - k0) * rstride;
             // softmax of the three logits, attention head lh (lanes >= H repeat head 0; nobody reads them)
@@ -609,7 +607,7 @@ __global__ void __launch_bounds__(kFrameThreads, 1) gat_aggregate_frame_kernel(A
         if (c == 0) init_acc();
 #pragma unroll
         for (int t = 0; t < kFrameOwn; ++t) {
-            while (hcur[t] < hdeg[t] && !(p.dbg & 32)) {
+            while (hcur[t] < hdeg[t]) {
                 const int pos = hbeg[t] + hcur[t];
                 const int kk = lsth[pos] - n0 - Hb;
                 if (kk >= k1) break;
@@ -670,7 +668,7 @@ __global__ void __launch_bounds__(kFrameThreads, 1) gat_aggregate_frame_kernel(A
 //   * the head rows arrive as ONE bulk copy (they are contiguous, a1|a2 tails included: no separate attention table);
 //   * row / plane addresses are formed once per destination, column offsets are immediates;
 //   * the K padding of the output planes is written by the lanes that idle in the last column group (no extra pass);
-//   * barrier waits poll without reading the clock; no debug switches, no fp32 side output (those take the generic kernel).
+//   * barrier waits poll without reading the clock; no fp32 side output (that takes the generic kernel).
 // ------------------------------------------------------------------------------------------------
 template <int H, int D> struct FrameShape {
     static constexpr int HD = H * D;
@@ -705,6 +703,7 @@ __device__ __forceinline__ void agg_mbar_wait_spin(uint32_t bar, uint32_t parity
     uint32_t done = 0, spins = 0;
     while (true) {
         // the hint lets the hardware park the warp for up to ~1 us instead of returning to the polling loop at once
+        // (the persistent kernel measured the same with hints from 0 to 100000 ns)
         asm volatile(
             "{\n\t.reg .pred p;\n\t"
             "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
@@ -1024,7 +1023,7 @@ __host__ __device__ inline FramePlanP frame_plan_p(int max_heads, int max_enodes
 // heads (5 views x 4 persons) - one head per warp balances part (b), and 22 warps hide the per-chunk latency chain
 // better than 18 - and 16 x 2 up to 32 heads (the register file holds 18 warps with two heads' accumulators each).
 template <int H, int D, bool L0, int W, int OWN>
-__global__ void __launch_bounds__((W + 2) * 32, 1) gat_aggregate_frame_p_kernel(AggParams p, int max_heads, int max_enodes, int slots, uint32_t hint)
+__global__ void __launch_bounds__((W + 2) * 32, 1) gat_aggregate_frame_p_kernel(AggParams p, int max_heads, int max_enodes, int slots)
 {
     using S = FrameShape<H, D>;
     constexpr int HD = S::HD, LDZ = S::LDZ, VEC = S::VEC, NV = S::NV, KMAX = S::KMAX, LDP = S::LDP, NVP = S::NVP;
@@ -1065,7 +1064,7 @@ __global__ void __launch_bounds__((W + 2) * 32, 1) gat_aggregate_frame_p_kernel(
             const int n_chunks = (Mb + W - 1) / W;
             for (int c = 0; c < n_chunks; ++c, ++g) {
                 const int s = g % slots;
-                if (g >= slots) agg_mbar_wait_spin(agg_smem_u32(&bar_empty[s]), (uint32_t)(g / slots - 1) & 1u, hint);
+                if (g >= slots) agg_mbar_wait_spin(agg_smem_u32(&bar_empty[s]), (uint32_t)(g / slots - 1) & 1u);
                 const int rows = min(W, Mb - c * W);
                 const uint32_t bytes = (uint32_t)rows * (uint32_t)(LDZ * 4);
                 const uint32_t bar = agg_smem_u32(&bar_full[s]);
@@ -1085,7 +1084,7 @@ __global__ void __launch_bounds__((W + 2) * 32, 1) gat_aggregate_frame_p_kernel(
             int* lsth = reinterpret_cast<int*>(set + f.lsth);
             int* prs = reinterpret_cast<int*>(set + f.prs);
             int* meta = reinterpret_cast<int*>(set + f.meta);
-            if (i >= 2) agg_mbar_wait_spin(agg_smem_u32(&bar_tab_empty[k]), (uint32_t)(i / 2 - 1) & 1u, hint);
+            if (i >= 2) agg_mbar_wait_spin(agg_smem_u32(&bar_tab_empty[k]), (uint32_t)(i / 2 - 1) & 1u);
             const int n0 = __ldg(p.node_off + b), Nb = __ldg(p.node_off + b + 1) - n0;
             const int h0 = __ldg(p.head_off + b), Hb = __ldg(p.head_off + b + 1) - h0;
             const int Mb = Nb - Hb, Eh = Hb + 2 * Mb, e0 = h0 + 5 * (n0 - h0);
@@ -1145,10 +1144,10 @@ __global__ void __launch_bounds__((W + 2) * 32, 1) gat_aggregate_frame_p_kernel(
         const int* lsth = reinterpret_cast<const int*>(set + f.lsth);
         const int* prs = reinterpret_cast<const int*>(set + f.prs);
         const int* meta = reinterpret_cast<const int*>(set + f.meta);
-        agg_mbar_wait_spin(agg_smem_u32(&bar_tab_full[ks]), (uint32_t)(i / 2) & 1u, hint);
+        agg_mbar_wait_spin(agg_smem_u32(&bar_tab_full[ks]), (uint32_t)(i / 2) & 1u);
         const int n0 = meta[0], Hb = meta[2], Mb = meta[3];
         if (Hb + Mb > 0) {
-            agg_mbar_wait_spin(agg_smem_u32(&bar_rows[ks]), (uint32_t)(i / 2) & 1u, hint);     // acquires the copied head rows
+            agg_mbar_wait_spin(agg_smem_u32(&bar_rows[ks]), (uint32_t)(i / 2) & 1u);     // acquires the copied head rows
             const int n_chunks = (Mb + W - 1) / W;
             // softmax weights of the heads' in-edges, per attention head (gat2.py:78-88): the consumers' own share, reported
             // through bar_wh; only part (b) below reads them, so nobody waits before its first edge-node destination is done
@@ -1184,7 +1183,7 @@ __global__ void __launch_bounds__((W + 2) * 32, 1) gat_aggregate_frame_p_kernel(
                 if (h < Hb) { hbeg[t] = meta[8 + 2 * h]; hdeg[t] = meta[8 + 2 * h + 1]; }
             }
             auto init_acc = [&]() {
-                agg_mbar_wait_spin(agg_smem_u32(&bar_wh[ks]), (uint32_t)(i / 2) & 1u, hint);
+                agg_mbar_wait_spin(agg_smem_u32(&bar_wh[ks]), (uint32_t)(i / 2) & 1u);
 #pragma unroll
                 for (int t = 0; t < OWN; ++t) {
                     const int h = wid + t * W;
@@ -1214,7 +1213,7 @@ __global__ void __launch_bounds__((W + 2) * 32, 1) gat_aggregate_frame_p_kernel(
                 int slot = 0;
                 if (!L0) {
                     slot = g % slots;
-                    agg_mbar_wait_spin(agg_smem_u32(&bar_full[slot]), (uint32_t)(g / slots) & 1u, hint);
+                    agg_mbar_wait_spin(agg_smem_u32(&bar_full[slot]), (uint32_t)(g / slots) & 1u);
                     rows = ring + (size_t)slot * W * LDZ;
                 }
                 // (a) the edge-node destination of this warp: in-edges (h1 -> e), (h2 -> e), (e -> e)
@@ -1475,7 +1474,7 @@ __global__ void __launch_bounds__(kAggWarps * 32, 2) gat_aggregate_large_kernel(
     if (u < p.edge_units) {
         // ---------------- edge-node destinations ----------------
         const int v_begin = Hb + u * kLargeChunk;
-        if (v_begin >= Nb || (p.dbg & 64)) return;
+        if (v_begin >= Nb) return;
         const int v_end = min(Nb, v_begin + kLargeChunk);
         float* zs = smem_l + plan.stage;
         const uint32_t zs_u32 = smem_base + 4u * plan.stage;
@@ -1618,7 +1617,6 @@ __global__ void __launch_bounds__(kAggWarps * 32, 2) gat_aggregate_large_kernel(
     }
 
     // ---------------- head destinations ----------------
-    if (p.dbg & 32) return;
     const int hh = warp / kWarpsPerHead, part_w = warp - hh * kWarpsPerHead;
     const int v = (u - p.edge_units) * kLargeHeads + hh;
     const uint32_t ring_u32 = smem_base + 4u * (plan.ring + warp * kHeadRing * ldz);
@@ -1804,7 +1802,6 @@ static int gat_aggregate_impl(int32_t n_frames, int32_t n_nodes_total, int32_t n
     p.act_hi = reinterpret_cast<__nv_bfloat16*>(act_hi); p.act_lo = reinterpret_cast<__nv_bfloat16*>(act_lo);
     p.ld_planes = ld_planes;
     p.res = res; p.ld_res = ld_res;
-    p.dbg = g_debug_flags;
     p.stage_cap = 0; p.edge_units = 0; p.head_units = 0;
     const int vec = (dim % 4 == 0) ? 4 : (dim % 2 == 0 ? 2 : 1);
     // A live frame or two (fewer frames than an eighth of the SMs): one CTA per frame would leave the GPU idle and pay one
@@ -1815,7 +1812,7 @@ static int gat_aggregate_impl(int32_t n_frames, int32_t n_nodes_total, int32_t n
     const bool frame_path = ((impl == 0 && !tiny_batch) || impl == 3 || impl == 5 || impl == 6) && max_heads_per_frame > 0 && max_enodes_per_frame > 0 &&
                             max_heads_per_frame <= kFrameOwn * kFrameWarps && HD / vec <= 32 * 4;
     // shape-specialised kernel (the shipped layer shapes, planes out, LeakyReLU slope in [0, 1]); impl 5 forces the generic one
-    if (frame_path && impl != 5 && act_hi && !raw_f32 && p.dbg == 0 && act_slope >= 0.f && act_slope <= 1.f && alpha >= 0.f && alpha <= 1.f) {
+    if (frame_path && impl != 5 && act_hi && !raw_f32 && act_slope >= 0.f && act_slope <= 1.f && alpha >= 0.f && alpha <= 1.f) {
         auto launch_s = [&](auto kern, const FramePlanS f, int ldz_s, int ldp_s, bool* taken) -> int {
             *taken = false;
             const size_t smem_s = (size_t)f.total_floats * sizeof(float);
@@ -1844,8 +1841,7 @@ static int gat_aggregate_impl(int32_t n_frames, int32_t n_nodes_total, int32_t n
             cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
             const int grid = n_frames < sms ? n_frames : sms;
             B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_p));
-            const uint32_t hint = 1000u;       // try_wait suspend hint [ns]; 0 .. 100000 measured the same
-            kern<<<grid, (warps + 2) * 32, smem_p, st>>>(p, max_heads_per_frame, max_enodes_per_frame, slots, hint);
+            kern<<<grid, (warps + 2) * 32, smem_p, st>>>(p, max_heads_per_frame, max_enodes_per_frame, slots);
             B2_CHECK_LAUNCH();
             return B200POSE_OK;
         };

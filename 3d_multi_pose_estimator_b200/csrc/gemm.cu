@@ -137,7 +137,6 @@ struct GemmParams2 {
     // fused second projection (b200pose_linear_fused2): out2[row, t] = sum_c act(out1)[row, c] * fuse_w[t, c] + fuse_b[t], t < fuse_n <= 4,
     // evaluated in the epilogue registers of a single n-tile; nothing of out1 is stored
     const float* fuse_w; const float* fuse_b; float* fuse_out; int fuse_n, fuse_ldw, fuse_ldo;
-    int dbg;                                 // kernel bring-up switches (b200pose_set_debug): 1 = no stores, 2 = hi*hi only, 4 = no epilogue math
 };
 
 struct TileInfo { int m0, n0, bn, n_eff; };   // n_eff: the tile's valid width rounded up to the MMA granule (16) - what is actually multiplied
@@ -351,10 +350,8 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_split_tc2_kernel(
                             umma_bf16(tmem_d, dah, dbl, idesc, 1u);
                         } else {
                             umma_bf16_pair(tmem_d, dah, dbh, idesc, first);
-                            if (!(p.dbg & 2)) {
-                                umma_bf16_pair(tmem_d, dal, dbh, idesc, 1u);
-                                umma_bf16_pair(tmem_d, dah, dbl, idesc, 1u);
-                            }
+                            umma_bf16_pair(tmem_d, dal, dbh, idesc, 1u);
+                            umma_bf16_pair(tmem_d, dah, dbl, idesc, 1u);
                         }
                     }
                     if constexpr (NCTA == 1) umma_commit(smem_u32(&bar_empty[s]));
@@ -397,7 +394,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_split_tc2_kernel(
                         else mbar_arrive_cluster(mapa_shared(smem_u32(&bar_acc_empty[a]), 0));
                     }
                 }
-                if (p.dbg & 4) continue;
                 float v[64];
                 // full panels with a 16-byte aligned bias: every lane reads the panel's 64 bias values with 16 broadcast
                 // vector loads (one L1 transaction each) instead of 128 shuffles - the epilogue warps share their
@@ -491,7 +487,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_split_tc2_kernel(
                     }
                     if (j == npanels - 1) {
                         const int row = t.m0 + (int)rank * kBM + q * 32 + lane;
-                        if (row < M_rows && !(p.dbg & 1)) {
+                        if (row < M_rows) {
                             for (int tt = 0; tt < p.fuse_n; ++tt) p.fuse_out[(size_t)row * p.fuse_ldo + tt] = facc[tt] + __ldg(p.fuse_b + tt);
                         }
                     }
@@ -526,7 +522,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_split_tc2_kernel(
                 __syncwarp();
                 if (lane == 0) {
                     const int row0 = t.m0 + (int)rank * kBM + q * 32;
-                    if (row0 < M_rows && !(p.dbg & 1)) {
+                    if (row0 < M_rows) {
                         if (p.has_f32) {
                             if (col0 < p.N) tma_store_2d(&map_o_f32, stage_f32, col0, row0);
                             if (col0 + 32 < p.N) tma_store_2d(&map_o_f32, stage_f32 + 4096u, col0 + 32, row0);
@@ -868,7 +864,7 @@ static int linear_impl(const uint16_t* a_hi, const uint16_t* a_lo, int32_t lda,
     const int ncta = (impl == 5) ? 2 : (impl == 4) ? 1 : (m > 4 * kBM ? 2 : 1);
     GemmParams2 q;
     q.M = m; q.N = n; q.num_kb = kpad / kBK; q.k_last = ceil_div(k - (kpad / kBK - 1) * kBK, kUmmaK); q.bias = bias; q.slope = slope; q.out_scale = out_scale;
-    q.has_f32 = out_f32 ? 1 : 0; q.has_planes = out_hi ? 1 : 0; q.dbg = g_debug_flags; q.m_dev = m_dev;
+    q.has_f32 = out_f32 ? 1 : 0; q.has_planes = out_hi ? 1 : 0; q.m_dev = m_dev;
     q.fuse_n = 0; q.fuse_w = nullptr; q.fuse_b = nullptr; q.fuse_out = nullptr; q.fuse_ldw = 0; q.fuse_ldo = 0;
     if (fuse) { q.fuse_n = fuse->n; q.fuse_w = fuse->w; q.fuse_b = fuse->b; q.fuse_out = fuse->out; q.fuse_ldw = fuse->ldw; q.fuse_ldo = fuse->ldo; }
     q.panels_total = ceil_div(n, 64);                         // 64-column panels; planes panels also zero columns [n, 64*panels)

@@ -156,10 +156,6 @@ int b200pose_linear_fused2(const uint16_t* a_hi, const uint16_t* a_lo, int32_t l
                            const float* w2_f32, int32_t ldw2, const float* bias2, int32_t n2,
                            float* out2_f32, int32_t ld_out2, void* stream);
 
-/* Kernel bring-up switches for the persistent GEMM (results become WRONG; used by scripts/gemm_probe.py to attribute time):
- * bit 0 = skip the output stores, bit 1 = issue only the hi*hi MMA, bit 2 = skip the epilogue arithmetic. Returns the old value. */
-int b200pose_set_debug(int flags);
-
 /* fp32 [rows, ld_in] -> planes [rows, ld_planes] (used once per weight matrix at load time, and by tests) */
 int b200pose_split_planes(const float* x, int32_t rows, int32_t cols, int32_t ld_in,
                           uint16_t* hi, uint16_t* lo, int32_t ld_planes, void* stream);
